@@ -1,8 +1,10 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the BP -> feedback-GNN -> BP hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+Every timed section runs K steps.
 
 Workload (BASELINE.json configs[2], named in config.workload): the [[1270,28]] GHP code, decoders
 (64, G, 16, G, 16, G, 16) with the shipped weights (the configuration of n1270.py / the reference's
@@ -170,20 +172,46 @@ def shared_config(B):
             "l2": "per-step working set (~23 KB/frame of HBM state, %d MB) exceeds the 126 MB L2" % (B * 23 // 1000)}
 
 
-def time_pipeline(ctx, comm, model, B, steps, warmup, allreduce=True):
+def time_pipeline(ctx, comm, model, B, steps, warmup, allreduce=True, keep_last=False):
     """`steps` passes of the whole pipeline, CUDA events on the context's stream, max over ranks.  One counter
-    all-reduce per step sits inside the timed region (the poll of sim_ber's stopping rule, misc.py:710-716)."""
+    all-reduce per step sits inside the timed region (the poll of sim_ber's stopping rule, misc.py:710-716).
+    With `keep_last` the last step also writes its per-frame outputs (flags, x_diff, z_diff), which only adds
+    stores to the final kernel, and returns them as the third value."""
     for _ in range(warmup):
         model.run(B, P_NOISE, want_flags=False, want_diff=False)
     comm.barrier()
     counters = np.zeros(4, np.int64)
+    last = None
     ctx.timer_start()
-    for _ in range(steps):
-        r = model.run(B, P_NOISE, want_flags=False, want_diff=False, want_counters=True)
+    for i in range(steps):
+        want = keep_last and i == steps - 1
+        r = model.run(B, P_NOISE, want_flags=want, want_diff=want, want_counters=True)
         counters = counters + (comm.allreduce_sum(r["counters"]) if allreduce else r["counters"])
+        if want:
+            last = r
     ms = ctx.timer_stop()
     comm.barrier()
-    return float(comm.allreduce_f64([ms], "max")[0]), counters
+    return float(comm.allreduce_f64([ms], "max")[0]), counters, last
+
+
+DUMP_FRAMES = 4096        # frames of the last step whose residuals are written (x_diff + z_diff: 41.6 MB in float32)
+
+
+def dump_outputs(path, res, first_frame, B):
+    """What the last timed step returned to its caller, as float32 / float64 .npy files: `counters` (frames, flagged,
+    block errors, stage-0 failures over the whole step) and, for a fixed seeded sample of its frames, `flags`
+    (bit 0 flagged, bit 1 block error, bits 2+ the stages before the last that left the frame active), `x_diff` /
+    `z_diff` (residual error: noise XOR correction, one row per frame) and `frames` (their global frame ids, which
+    key the in-kernel noise)."""
+    os.makedirs(path, exist_ok=True)
+    rows = np.sort(np.random.default_rng(0).choice(B, size=min(B, DUMP_FRAMES), replace=False))
+    out = {"counters": res["counters"].astype(np.float64),
+           "frames": (first_frame + rows).astype(np.float64),
+           "flags": res["flags"].numpy()[rows].astype(np.float32),
+           "x_diff": res["x_diff"].numpy()[rows].astype(np.float32),
+           "z_diff": res["z_diff"].numpy()[rows].astype(np.float32)}
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def main():
@@ -201,7 +229,12 @@ def main():
                     help="arithmetic of the headline: exp/log on the SFU (default) or as FP32 polynomials; both are "
                          "bit-exact against the CPU oracle in the same arithmetic (csrc/fb_math.h)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline returned (rank 0) to DIR/<name>.npy, so that two "
+                         "builds can be compared output for output; the same arguments give the same inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -235,30 +268,33 @@ def main():
     if rank == 0:
         sampler.start()
     launches0 = ctx.launch_count()
-    ms, counters = time_pipeline(ctx, comm, model, B, args.steps, 0)
+    dump = args.dump_outputs is not None and rank == 0
+    ms, counters, last = time_pipeline(ctx, comm, model, B, args.steps, 0, keep_last=dump)
     launches = ctx.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
     bp_frames, bp_iters = ctx.stats(reset=True)
     value = args.steps * B * world / (ms * 1e-3)
+    if dump:
+        dump_outputs(args.dump_outputs, last, model.next_frame - B, B)
 
     # ---- the other arithmetic on the same workload, reported beside the headline
     ctx.set_math(other)
-    o_steps = max(3, min(args.steps, 5))
-    o_ms, o_counters = time_pipeline(ctx, comm, model, B, o_steps, 2)
+    o_steps = args.steps
+    o_ms, o_counters, _ = time_pipeline(ctx, comm, model, B, o_steps, 2)
     o_value = o_steps * B * world / (o_ms * 1e-3)
     ctx.set_math(args.math)
 
     # ---- the same workload with round skipping (result-identical; what low-p sweeps use)
     model.skip_inactive = True
-    s_steps = max(3, min(args.steps, 5))
-    s_ms, s_counters = time_pipeline(ctx, comm, model, B, s_steps, 2)
+    s_steps = args.steps
+    s_ms, s_counters, _ = time_pipeline(ctx, comm, model, B, s_steps, 2)
     model.skip_inactive = False
     s_value = s_steps * B * world / (s_ms * 1e-3)
 
     # ---- the same workload with the other evaluation of the feedback GNN's dense products (tensor cores <-> FP32 FMAs)
     tc_model = build_model(code, seed=2, first_frame=rank * per_rank_frames, gemm=other_gemm)
-    t_steps = max(3, min(args.steps, 5))
-    t_ms, t_counters = time_pipeline(ctx, comm, tc_model, B, t_steps, 2)
+    t_steps = args.steps
+    t_ms, t_counters, _ = time_pipeline(ctx, comm, tc_model, B, t_steps, 2)
     t_value = t_steps * B * world / (t_ms * 1e-3)
 
     # ---- end to end through the public API with HOST buffers: packed noise bit-planes in, packed indicator planes out
@@ -286,7 +322,7 @@ def main():
     comm.barrier()
     t0 = time.perf_counter()
     ctx.timer_start()
-    e2e_steps = max(3, min(args.steps, 5))
+    e2e_steps = args.steps
     for _ in range(e2e_steps):
         blk, c = e2e_step()
         assert blk == c[2]

@@ -105,7 +105,7 @@ def main():
         rng = np.random.default_rng(3)
         prior = np.float32(np.log(np.float64(np.float32(3. * (1. - 0.05) / 0.05))))
         llr = (prior + rng.normal(0, 0.3, (B, 3, code.N))).astype(np.float32)
-        bp[f"{cname}.noise_x"], bp[f"{cname}.noise_z"], bp[f"{cname}.u"] = nx, nz, u
+        bp[f"{cname}.noise_x"], bp[f"{cname}.noise_z"] = nx, nz
         bp[f"{cname}.llr"], bp[f"{cname}.sx"], bp[f"{cname}.sz"] = llr, sx.astype(np.uint8), sz.astype(np.uint8)
         bp[f"{cname}.p"] = np.float64(p)
         for cn_type, factor, iters in cases:
@@ -129,7 +129,10 @@ def main():
                                     cn_type="boxplus-phi", trainable=True)
             llr_hat, xh, zh = dec((tf.constant(llr[:4]), tf.constant(sx[:, :4]), tf.constant(sz[:, :4])))
             bp["c882.trainable.llr_hat"] = np.asarray(llr_hat)
-    np.savez_compressed(os.path.join(HERE, "ref_bp4.npz"), **bp)
+    # two files, so that each stays under 1 MB
+    np.savez_compressed(os.path.join(HERE, "ref_bp4.npz"), **{k: v for k, v in bp.items() if k.startswith("c882.")})
+    np.savez_compressed(os.path.join(HERE, "ref_bp4_c1270_rsurf3.npz"),
+                        **{k: v for k, v in bp.items() if not k.startswith("c882.")})
 
     # ---------------------------------------------------------------- 2b. LDPCBPDecoder.call, is_syndrome (decoding.py:875-1048)
     from oracle import c_oracle as O

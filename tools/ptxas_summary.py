@@ -1,6 +1,8 @@
-"""Summarise registers / spills per kernel from the nvcc -Xptxas -v log (development aid)."""
-import re, sys
-log = open(sys.argv[1] if len(sys.argv) > 1 else "feedback-gnn_b200/csrc/build.log").read()
+"""Summarise registers / spills per kernel from the nvcc -Xptxas -v logs (development aid); by default the per-unit
+logs the build leaves in feedback-gnn_b200/csrc/_build/."""
+import glob, re, sys
+paths = sys.argv[1:] or sorted(glob.glob("feedback-gnn_b200/csrc/_build/*.log"))
+log = "".join(open(p).read() for p in paths)
 cur = None
 for line in log.splitlines():
     m = re.search(r"Compiling entry function '(\S+)'", line)
