@@ -131,4 +131,4 @@ void ws_free(Workspace &w);                                              // fbgn
 int launch_bp4(fbgnn_ctx *ctx, const Bp4Args &a, int64_t grid);          // fbgnn_bp.cu
 int launch_bp2(fbgnn_ctx *ctx, const Bp2Args &a, int64_t B);             // fbgnn_bp.cu
 int launch_gnn(fbgnn_ctx *ctx, const fbgnn_gnn *g, GnnArgs &a);          // fbgnn_gnn.cu
-int launch_osd0(fbgnn_ctx *ctx, Osd0Args &a, int64_t grid);              // fbgnn_pipeline.cu
+int launch_osd(fbgnn_ctx *ctx, OsdArgs &a, int order, int64_t grid);    // fbgnn_pipeline.cu

@@ -2064,14 +2064,19 @@ static __global__ void k_syndrome(const SyndromeArgs a) {
     }
 }
 
-// ------------------------------------------------------------------ OSD-0 -------------
+// ------------------------------------------------------------------ OSD ---------------
 // OSD0_Decoder (bp_osd.py:8-77) for the frames BP left with a syndrome mismatch: order the columns
 // by increasing reliability (stable), then for every row of the full-rank basis take the first
-// remaining one as pivot and eliminate it from all other rows of [H_perm | s]; the solution sits on
-// the pivot columns.  One CTA per frame; the permuted bit matrix lives in shared memory, stored
+// remaining one as pivot and eliminate it from all other rows of [H_perm | s]; the OSD-0 solution
+// sits on the pivot columns.  One CTA per frame; the permuted bit matrix lives in shared memory, stored
 // word-major (M[w * Rp + row]) so that the row-parallel XOR sweeps are conflict-free and the pivot
 // row is a broadcast.
-struct Osd0Args {
+// With order lam > 0 the combination sweep (OSD-CS, Roffe et al. 2020) runs on that reduced matrix
+// before it is discarded.  Over the non-pivot columns c_0 < c_1 < ... (least reliable first) the
+// candidates T are, by index: 0 the empty set (OSD-0), 1 + i the single {c_i}, then the pairs
+// {c_i, c_j}, i < j < min(lam, n - R), in lexicographic order.  T's solution is 1 on T and
+// s'_r ^ XOR_{c in T} M[r, c] on pivot piv[r]; the candidate of least (Hamming weight, index) wins.
+struct OsdArgs {
     SideDev S;                          // graph of the basis matrix: rows = the rank basis rows
     const int *frame_list;              // optional: CTA i handles frame frame_list[i]
     View2<const float> llr;             // (b, v) reliabilities; the sort key is sign * llr
@@ -2081,7 +2086,9 @@ struct Osd0Args {
     View2<uint8_t> e_hat;               // (b, v) optional output
     uint8_t *vbits;                     // optional [B][n]: the solution goes to bit `vbit` (pipeline mode)
     int vbit;
+    int order;                          // 0: OSD-0; lam > 0: OSD-CS of order lam
     int npad;                           // power of two >= n
+    int cv_off;                         // byte offset of the OSD-CS bit vectors in shared memory (order > 0)
 };
 
 __device__ __forceinline__ unsigned long long osd_key(float x, int idx) {
@@ -2090,8 +2097,20 @@ __device__ __forceinline__ unsigned long long osd_key(float x, int idx) {
     return ((unsigned long long)u << 32) | (uint32_t)idx;
 }
 
-// smem: max(npad * 8, W * Rp * 4) bytes shared by the sort keys and the matrix; u16 order[n], inv[n], piv[R]
-static __global__ void __launch_bounds__(256) k_osd0(const Osd0Args a) {
+// pair q (lexicographic over i < j < lp) -> (i, j); row i of the triangle starts at i (2 lp - i - 1) / 2
+__device__ __forceinline__ void osd_pair(int64_t q, int lp, int &i, int &j) {
+    const double t = 2.0 * lp - 1.0;
+    i = (int)((t - sqrt(t * t - 8.0 * (double)q)) * 0.5);
+    i = max(0, min(i, lp - 2));
+    auto start = [lp](int r) { return (int64_t)r * (2 * lp - r - 1) / 2; };
+    while (i > 0 && start(i) > q) i--;
+    while (i < lp - 2 && start(i + 1) <= q) i++;
+    j = (int)(i + 1 + (q - start(i)));
+}
+
+// smem: max(npad * 8, W * Rp * 4) bytes shared by the sort keys and the matrix; u16 order[n], inv[n], piv[R];
+// with order > 0, at cv_off: u32 cv[lp][RW] (the first lp non-pivot columns over the rows) and sv[RW] (s')
+static __global__ void __launch_bounds__(256) k_osd(const OsdArgs a) {
     extern __shared__ unsigned long long osd_smem[];
     const SideDev &S = a.S;
     const int n = S.n, R = S.m, T = blockDim.x, tid = threadIdx.x;
@@ -2173,14 +2192,98 @@ static __global__ void __launch_bounds__(256) k_osd0(const Osd0Args a) {
         __syncthreads();
     }
 
-    // 4. solution on the pivot columns, mapped back through the permutation
+    // 4. OSD-CS: the candidate of least (weight, index); t0 / t1 are its columns (-1: none)
+    int t0 = -1, t1 = -1;
+    if (a.order > 0) {
+        __shared__ unsigned long long best;
+        __shared__ int num_np;
+        const int RW = (R + 31) / 32, lp = min(a.order, max(n - R, 0));
+        const int lane = tid & 31, warp = tid >> 5, nw = T >> 5;
+        uint32_t *cv = (uint32_t *)((uint8_t *)osd_smem + a.cv_off), *sv = cv + (size_t)lp * RW;
+        // 4a. the non-pivot columns in increasing position, listed in inv (free since step 2); s' as a bit vector
+        for (int j = tid; j < n; j += T) inv[j] = 1;
+        if (tid == 0) best = ~0ull;
+        __syncthreads();
+        for (int r = tid; r < R; r += T) inv[piv[r]] = 0;
+        __syncthreads();
+        if (warp == 0) {
+            int cnt = 0;
+            for (int j0 = 0; j0 < n; j0 += 32) {                   // list position <= column: reads stay ahead of writes
+                const int j = j0 + lane;
+                const bool np_col = j < n && inv[j];
+                const uint32_t vote = __ballot_sync(0xffffffffu, np_col);
+                if (np_col) inv[cnt + __popc(vote & ((1u << lane) - 1u))] = (uint16_t)j;
+                cnt += __popc(vote);
+            }
+            if (lane == 0) num_np = cnt;
+        }
+        for (int k = warp; k < RW; k += nw) {
+            const int r = k * 32 + lane;
+            const uint32_t v = __ballot_sync(0xffffffffu, r < R && ((M[wn * Rp + r] >> (n & 31)) & 1u));
+            if (lane == 0) sv[k] = v;
+        }
+        __syncthreads();
+        const int N = num_np;
+        unsigned long long mine = ~0ull;
+        if (tid == 0) {                                            // the empty set: OSD-0
+            int w = 0;
+            for (int k = 0; k < RW; k++) w += __popc(sv[k]);
+            mine = (unsigned long long)w << 32;
+        }
+        // 4b. single columns: a warp ballots 32 rows at a time (conflict-free) and keeps the first lp as bit vectors
+        for (int i = warp; i < N; i += nw) {
+            const int c = inv[i], cw = c >> 5;
+            const uint32_t cm = 1u << (c & 31);
+            int w = 1;
+            for (int k = 0; k < RW; k++) {
+                const int r = k * 32 + lane;
+                const uint32_t v = __ballot_sync(0xffffffffu, r < R && (M[cw * Rp + r] & cm));
+                if (i < lp && lane == 0) cv[i * RW + k] = v;
+                w += __popc(v ^ sv[k]);
+            }
+            if (lane == 0) mine = min(mine, ((unsigned long long)w << 32) | (uint32_t)(1 + i));
+        }
+        __syncthreads();
+        // 4c. pairs of the first lp columns, one thread per pair
+        const int64_t P = (int64_t)lp * (lp - 1) / 2;
+        for (int64_t q = tid; q < P; q += T) {
+            int i, j;
+            osd_pair(q, lp, i, j);
+            int w = 2;
+            for (int k = 0; k < RW; k++) w += __popc(sv[k] ^ cv[i * RW + k] ^ cv[j * RW + k]);
+            mine = min(mine, ((unsigned long long)w << 32) | (uint32_t)(1 + N + q));
+        }
+        for (int o = 16; o > 0; o >>= 1) mine = min(mine, __shfl_xor_sync(0xffffffffu, mine, o));
+        if (lane == 0) atomicMin(&best, mine);
+        __syncthreads();
+        const uint32_t idx = (uint32_t)best;
+        if (idx >= 1 && idx <= (uint32_t)N) t0 = inv[idx - 1];
+        else if (idx > (uint32_t)N) {
+            int i, j;
+            osd_pair((int64_t)idx - 1 - N, lp, i, j);
+            t0 = inv[i]; t1 = inv[j];
+        }
+    }
+
+    // 5. the solution on the pivot columns and on T, mapped back through the permutation
     if (a.e_hat.ptr) for (int v = tid; v < n; v += T) a.e_hat(b, v) = 0;
     if (a.vbits) for (int v = tid; v < n; v += T) a.vbits[b * n + v] &= (uint8_t)~(1u << a.vbit);
     __syncthreads();
     for (int r = tid; r < R; r += T) {
-        const int sol = (M[wn * Rp + r] >> (n & 31)) & 1u;
+        int sol = (M[wn * Rp + r] >> (n & 31)) & 1u;
+        if (t0 >= 0) sol ^= (M[(t0 >> 5) * Rp + r] >> (t0 & 31)) & 1u;
+        if (t1 >= 0) sol ^= (M[(t1 >> 5) * Rp + r] >> (t1 & 31)) & 1u;
         const int v = order[piv[r]];
         if (sol) {
+            if (a.e_hat.ptr) a.e_hat(b, v) = 1;
+            if (a.vbits) a.vbits[b * n + v] |= (uint8_t)(1u << a.vbit);
+        }
+    }
+    if (tid == 0) {
+        for (int e = 0; e < 2; e++) {
+            const int c = e ? t1 : t0;
+            if (c < 0) continue;
+            const int v = order[c];
             if (a.e_hat.ptr) a.e_hat(b, v) = 1;
             if (a.vbits) a.vbits[b * n + v] |= (uint8_t)(1u << a.vbit);
         }

@@ -1,34 +1,53 @@
-// fbgnn_pipeline.cu -- the fused Monte-Carlo pipelines (multi-launch orchestration) and OSD-0.
+// fbgnn_pipeline.cu -- the fused Monte-Carlo pipelines (multi-launch orchestration) and OSD.
 #include "fbgnn_internal.h"
 
-// ------------------------------------------------------------------ OSD-0 ---------------
-int launch_osd0(fbgnn_ctx *ctx, Osd0Args &a, int64_t grid) {
+// ------------------------------------------------------------------ OSD -----------------
+int launch_osd(fbgnn_ctx *ctx, OsdArgs &a, int order, int64_t grid) {
     if (grid <= 0) return 0;
     const int n = a.S.n, R = a.S.m, W = (n + 1 + 31) / 32, Rp = R | 1;
     int npad = 1;
     while (npad < n) npad <<= 1;
     a.npad = npad;
+    a.order = order;
     const size_t main_bytes = std::max<size_t>((size_t)npad * 8, (size_t)W * Rp * 4);
-    const size_t smem = ((main_bytes + 7) & ~(size_t)7) + sizeof(uint16_t) * (2 * (size_t)n + R) + 16;
-    if (int rc = set_smem(k_osd0, smem, ctx, "OSD-0")) return rc;
-    k_osd0<<<(unsigned)grid, 256, smem, ctx->stream>>>(a);
+    const size_t u16_bytes = sizeof(uint16_t) * (2 * (size_t)n + R);
+    size_t smem = ((main_bytes + 7) & ~(size_t)7) + u16_bytes + 16;
+    if (order > 0) {            // OSD-CS: the first lp non-pivot columns and s' as ceil(R/32)-word bit vectors
+        const size_t lp = (size_t)std::min(order, std::max(n - R, 0)), RW = ((size_t)R + 31) / 32;
+        a.cv_off = (int)(((main_bytes + 7) & ~(size_t)7) + ((u16_bytes + 15) & ~(size_t)15));
+        smem = (size_t)a.cv_off + (lp + 1) * RW * 4;
+    }
+    if (int rc = set_smem(k_osd, smem, ctx, order > 0 ? "OSD-CS" : "OSD-0")) return rc;
+    k_osd<<<(unsigned)grid, 256, smem, ctx->stream>>>(a);
     CK(cudaGetLastError());
     ctx->launches++;
     return 0;
 }
 
-extern "C" int fbgnn_osd0_decode(fbgnn_graph *basis, int64_t B, fbgnn_tensor2 llr, fbgnn_tensor2 synd,
-                                 fbgnn_tensor2 e_hat) {
+// OSD-CS candidate indices are 32-bit: 1 + N + lp (lp - 1) / 2 < 2^32 for lp <= 65535
+static int check_osd_order(int32_t order) {
+    REQUIRE(order >= 0 && order <= 65535, "OSD order %d outside [0, 65535]", order);
+    return 0;
+}
+
+extern "C" int fbgnn_osd_decode(fbgnn_graph *basis, int32_t order, int64_t B, fbgnn_tensor2 llr, fbgnn_tensor2 synd,
+                                fbgnn_tensor2 e_hat) {
     REQUIRE(basis && llr.ptr && synd.ptr && e_hat.ptr && B >= 0, "bad argument");
+    if (int rc = check_osd_order(order)) return rc;
     if (int rc = need_decodable(basis)) return rc;
     fbgnn_ctx *ctx = basis->ctx;
     if (set_device(ctx)) return FBGNN_E_CUDA;
-    Osd0Args a{};
+    OsdArgs a{};
     a.S = basis->dev;
     a.llr = v2<const float>(llr); a.sign = 1.0f;
     a.synd = v2<const uint8_t>(synd);
     a.e_hat = v2<uint8_t>(e_hat);
-    return launch_osd0(ctx, a, B);
+    return launch_osd(ctx, a, order, B);
+}
+
+extern "C" int fbgnn_osd0_decode(fbgnn_graph *basis, int64_t B, fbgnn_tensor2 llr, fbgnn_tensor2 synd,
+                                 fbgnn_tensor2 e_hat) {
+    return fbgnn_osd_decode(basis, 0, B, llr, synd, e_hat);
 }
 
 // ------------------------------------------------------------------ pipelines -----------
@@ -93,6 +112,7 @@ static int pipeline_run_impl(fbgnn_code *code, const fbgnn_pipeline_cfg *cfg, ui
     REQUIRE((noise_x.ptr == nullptr) == (noise_z.ptr == nullptr), "give both noise_x and noise_z or neither");
     REQUIRE(B >= 0 && B < ((int64_t)1 << 31), "bad batch size");
     REQUIRE(!cfg->osd0 || (code->basis_x && code->basis_z), "OSD-0 needs fbgnn_code_set_basis first");
+    if (int rc = check_osd_order(cfg->osd_order)) return rc;
     REQUIRE(cfg->fixed_weight <= 0 || code->X->dev.n <= 65535, "fixed-weight sampling shuffles uint16 qubit indices (n <= 65535)");
     for (int s = 0; s < cfg->num_stages; s++) {
         REQUIRE(cfg->cn_type[s] >= 0 && cfg->cn_type[s] <= 2, "unknown cn_type in stage %d", s);
@@ -193,17 +213,17 @@ static int pipeline_run_impl(fbgnn_code *code, const fbgnn_pipeline_cfg *cfg, ui
         else k_osd_llr<MathExact><<<(unsigned)blocks, 256, 0, st>>>(la);
         CK(cudaGetLastError());
         ctx->launches++;
-        Osd0Args oa{};
+        OsdArgs oa{};
         oa.frame_list = cur_list; oa.sign = 1.0f;
         oa.vbits = w.vbits;
         oa.S = code->basis_x->dev;                                   // hx basis, osd_llrz, syndrome_x -> z_hat
         oa.llr = View2<const float>{w.P + np, 3 * (int64_t)np, 1};
         oa.synd = View2<const uint8_t>{w.sbits, 1, mp}; oa.synd_row = code->pivot_x; oa.vbit = 3;
-        if (int rc = launch_osd0(ctx, oa, cur_count)) return rc;
+        if (int rc = launch_osd(ctx, oa, cfg->osd_order, cur_count)) return rc;
         oa.S = code->basis_z->dev;                                   // hz basis, osd_llrx, syndrome_z -> x_hat
         oa.llr = View2<const float>{w.P, 3 * (int64_t)np, 1};
         oa.synd = View2<const uint8_t>{w.sbits + X.m, 1, mp}; oa.synd_row = code->pivot_z; oa.vbit = 2;
-        if (int rc = launch_osd0(ctx, oa, cur_count)) return rc;
+        if (int rc = launch_osd(ctx, oa, cfg->osd_order, cur_count)) return rc;
     }
 
     FinalArgs fa{};
@@ -235,7 +255,16 @@ extern "C" int fbgnn_bsc_pipeline_run(fbgnn_graph *g, fbgnn_graph *logical, int3
                                       float factor, float llr_const, float p, uint64_t seed, uint64_t first_frame,
                                       int64_t B, fbgnn_tensor2 noise, uint8_t *flags, int64_t *counters,
                                       fbgnn_graph *osd_basis, const int32_t *osd_pivot) {
+    return fbgnn_bsc_pipeline_run_ex(g, logical, cn_type, num_iter, factor, llr_const, p, seed, first_frame, B, noise,
+                                     flags, counters, osd_basis, osd_pivot, 0);
+}
+
+extern "C" int fbgnn_bsc_pipeline_run_ex(fbgnn_graph *g, fbgnn_graph *logical, int32_t cn_type, int32_t num_iter,
+                                         float factor, float llr_const, float p, uint64_t seed, uint64_t first_frame,
+                                         int64_t B, fbgnn_tensor2 noise, uint8_t *flags, int64_t *counters,
+                                         fbgnn_graph *osd_basis, const int32_t *osd_pivot, int32_t osd_order) {
     REQUIRE(g, "graph is NULL");
+    if (int rc = check_osd_order(osd_order)) return rc;
     REQUIRE(!osd_basis || (osd_pivot && osd_basis->dev.n == g->dev.n && osd_basis->dev.m <= g->dev.m),
             "bad OSD-0 basis");
     REQUIRE(cn_type >= 0 && cn_type <= 2, "unknown cn_type %d", cn_type);
@@ -289,12 +318,12 @@ extern "C" int fbgnn_bsc_pipeline_run(fbgnn_graph *g, fbgnn_graph *logical, int3
             idx_t *dp = nullptr;
             CK(cudaMallocAsync(&dp, R * sizeof(idx_t), st));
             CK(cudaMemcpyAsync(dp, piv.data(), R * sizeof(idx_t), cudaMemcpyHostToDevice, st));
-            Osd0Args oa{};
+            OsdArgs oa{};
             oa.S = osd_basis->dev; oa.frame_list = w.list[0];
             oa.llr = View2<const float>{w.L, n, 1}; oa.sign = -1.0f;      // llr_hat = -decoder output
             oa.synd = View2<const uint8_t>{w.sbits, 1, mp}; oa.synd_row = dp;
             oa.vbits = w.vbits; oa.vbit = 2;
-            if (int rc = launch_osd0(ctx, oa, cnt)) return rc;
+            if (int rc = launch_osd(ctx, oa, osd_order, cnt)) return rc;
             CK(cudaStreamSynchronize(st));                                  // piv must outlive the copy
             CK(cudaFreeAsync(dp, st));
         }

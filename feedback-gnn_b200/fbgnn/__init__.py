@@ -16,7 +16,7 @@ from .decoding import LDPCBPDecoder
 from .pauli import Pauli, pauli_thresholds
 from .feedback_gnn import (Feedback_GNN, Sandwich_BP_GNN_Evaluation_Model, BP_BSC_Model, ErrorIndicator, pack_bits,
                            unpack_bits, packed_words)
-from .bp_osd import OSD0_Decoder, BP4_OSD_Model, BP2_OSD_Model
+from .bp_osd import OSD_Decoder, OSD0_Decoder, BP4_OSD_Model, BP2_OSD_Model
 from .utils import count_block_errors, count_errors, compute_bler, compute_ber, zeros_like, sim_ber, PlotBER, BinarySource
 from .training import (First_Stage_BP_Model, Second_Stage_GNN_BP_Model, Adam, CosineDecay, clip_by_value, train_step,
                        BP4_Error_Model, Feedback_GNN_Error_Model)

@@ -1,4 +1,4 @@
-"""BP + OSD-0 post-processing -- ``OSD0_Decoder``, ``BP4_OSD_Model``, ``BP2_OSD_Model``.
+"""BP + OSD post-processing -- ``OSD_Decoder``, ``OSD0_Decoder``, ``BP4_OSD_Model``, ``BP2_OSD_Model``.
 
 Mirrors ``sionna/fec/ldpc/bp_osd.py`` of the reference: the frames whose BP decision misses the
 syndrome are re-solved by ordered-statistics decoding of order 0 (``:8-77``): columns ordered by the
@@ -6,7 +6,12 @@ reliabilities BP produced, row-wise Gaussian elimination of the full-rank basis 
 solution on the pivot columns.  The models keep the reference's contract: ``model(batch_size, p)``
 returns ``(zeros_like(ls_hat), ls_hat)`` with ``ls_hat`` the logical-operator parities of the
 residual error (``:183-197``, ``:262-274``), so ``PlotBER.simulate(..., qldpc=False)`` counts block
-errors from it.  Everything runs on the GPU (``k_osd0`` and the fused pipelines).
+errors from it.  Everything runs on the GPU (``k_osd`` and the fused pipelines).
+
+``OSD_Decoder(n, osd_order=λ)`` adds the combination sweep of Roffe et al., "Decoding across the quantum LDPC code
+landscape" (2020) -- the ``ldpc`` package's ``osd_method="osd_cs"`` -- on the matrix OSD-0 has reduced: every single
+non-pivot column, then every pair of the first λ non-pivot columns (least reliable first), each flipped on top of the
+OSD-0 solution; the lightest solution (Hamming weight, ties to the earlier candidate) is returned.  Order 0 is OSD-0.
 
 Ties between equal reliabilities are broken by qubit index (the reference's ``tf.argsort`` leaves
 them to the backend).
@@ -19,11 +24,23 @@ from .decoding_q import QLDPCBPDecoder, _is_device, _to_u8
 from .feedback_gnn import BP_BSC_Model, ErrorIndicator, Sandwich_BP_GNN_Evaluation_Model
 
 
-class OSD0_Decoder:
-    """``OSD0_Decoder(n)(llr [bs,n], pcm [bs,rank,n] or [rank,n], s [rank,bs], bs) -> e_hat [bs,n]`` bool."""
+OSD_METHODS = ("osd0", "osd_cs")
 
-    def __init__(self, n, ctx=None):
+
+class OSD_Decoder:
+    """``OSD_Decoder(n, osd_order=0, osd_method="osd_cs")(llr [bs,n], pcm [bs,rank,n] or [rank,n], s [rank,bs], bs)
+    -> e_hat [bs,n]`` bool.  ``osd_method="osd0"`` or ``osd_order=0``: OSD-0; otherwise OSD-CS of order
+    ``osd_order`` (at most 65535)."""
+
+    def __init__(self, n, osd_order=0, osd_method="osd_cs", ctx=None):
+        if osd_method not in OSD_METHODS:
+            raise ValueError(f"osd_method must be one of {OSD_METHODS}, got {osd_method!r}")
+        osd_order = int(osd_order)
+        if not 0 <= osd_order <= 65535:
+            raise ValueError(f"osd_order must be in [0, 65535], got {osd_order}")
         self.n = int(n)
+        self.osd_method = osd_method
+        self.osd_order = 0 if osd_method == "osd0" else osd_order
         self._ctx = ctx
         self._graphs = {}
 
@@ -46,10 +63,21 @@ class OSD0_Decoder:
         if llr_d.shape != (B, self.n) or g.n != self.n or s_d.shape != (g.m, B):
             raise ValueError(f"expected llr [bs,{self.n}], pcm [rank,{self.n}], s [rank,bs]")
         e_hat = ctx.empty((B, self.n), np.uint8)
-        _ffi.call("fbgnn_osd0_decode", g.handle, B, llr_d.t2(), s_d.t2(), e_hat.t2())
+        _ffi.call("fbgnn_osd_decode", g.handle, self.osd_order, B, llr_d.t2(), s_d.t2(), e_hat.t2())
         return e_hat if on_device else e_hat.numpy().astype(bool)
 
     call = __call__
+
+
+class OSD0_Decoder(OSD_Decoder):
+    """``OSD0_Decoder(n)``: ``OSD_Decoder`` of order 0 (bp_osd.py:8-77)."""
+
+    def __init__(self, n, ctx=None):
+        super().__init__(n, osd_order=0, osd_method="osd0", ctx=ctx)
+
+
+def _osd_order(osd_decoder):
+    return int(getattr(osd_decoder, "osd_order", 0))
 
 
 def _indicators(flags, rows, dense=None):
@@ -69,8 +97,8 @@ def _indicators(flags, rows, dense=None):
 
 
 class BP4_OSD_Model:
-    """Quaternary BP followed by OSD-0 on the failed frames (bp_osd.py:80-197).  The prior is
-    log(3(1-p)/p) with the simulated p (``:121``)."""
+    """Quaternary BP followed by OSD on the failed frames (bp_osd.py:80-197), of the order of ``osd_decoder``
+    (``OSD0_Decoder``: OSD-0).  The prior is log(3(1-p)/p) with the simulated p (``:121``)."""
 
     def __init__(self, code, bp4_decoder, osd_decoder, seed=0, first_frame=0, ctx=None):
         if not isinstance(bp4_decoder, QLDPCBPDecoder):
@@ -78,7 +106,8 @@ class BP4_OSD_Model:
         self.code, self.k, self.n = code, code.K, code.N
         self.bp4_decoder, self.osd_decoder = bp4_decoder, osd_decoder
         self._inner = Sandwich_BP_GNN_Evaluation_Model(code, [bp4_decoder], [], num_layers=1, p0=None, seed=seed,
-                                                       first_frame=first_frame, osd0=True, ctx=ctx)
+                                                       first_frame=first_frame, osd0=True,
+                                                       osd_order=_osd_order(osd_decoder), ctx=ctx)
 
     @property
     def last_counters(self):
@@ -101,8 +130,8 @@ class BP4_OSD_Model:
 
 
 class BP2_OSD_Model:
-    """Binary syndrome BP on a BSC followed by OSD-0 on the failed frames (bp_osd.py:199-274);
-    the BP logit is -log((1-p)/p) with the simulated p (``:221``)."""
+    """Binary syndrome BP on a BSC followed by OSD on the failed frames (bp_osd.py:199-274), of the order of
+    ``osd_decoder``; the BP logit is -log((1-p)/p) with the simulated p (``:221``)."""
 
     def __init__(self, pcm, pcm_basis, pivot_pcm, logical_pcm, bp2_decoder, osd_decoder, seed=0, first_frame=0,
                  ctx=None):
@@ -128,6 +157,7 @@ class BP2_OSD_Model:
             g, _ = inner._graphs()
             inner._osd_basis = _ffi.Graph(self.pcm_basis, g.ctx)
             inner._osd_pivot = self.pivot_pcm
+            inner._osd_order = _osd_order(self.osd_decoder)
         return inner.run(batch_size, p, **kw)
 
     def __call__(self, batch_size, ebno_db):

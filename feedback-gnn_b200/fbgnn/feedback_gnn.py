@@ -264,10 +264,11 @@ class Sandwich_BP_GNN_Evaluation_Model:
       early_stop      opt-in: every BP stage leaves a frame's iteration loop at the first iteration whose decision
                       reproduces the syndrome (SURVEY.md H8).  NOT what the reference computes -- it always runs
                       num_iter iterations -- so it is off by default and excluded from parity claims
+      osd_order       with osd0: 0 runs OSD-0, λ > 0 the combination sweep OSD-CS of order λ (bp_osd.OSD_Decoder)
     """
 
     def __init__(self, code, decoders, feedbacks, num_layers=4, wt=False, p0=0.05, seed=0, first_frame=0,
-                 skip_inactive=False, osd0=False, ctx=None, early_stop=False):
+                 skip_inactive=False, osd0=False, ctx=None, early_stop=False, osd_order=0):
         self.k, self.n = code.K, code.N
         self.code = code
         self.hx, self.hz, self.lx, self.lz = code.hx, code.hz, code.lx, code.lz
@@ -295,6 +296,9 @@ class Sandwich_BP_GNN_Evaluation_Model:
         self.skip_inactive = bool(skip_inactive)
         self.osd0 = bool(osd0)          # OSD-0 on the frames the last BP stage leaves mismatching (bp_osd.py)
         self.early_stop = bool(early_stop)   # opt-in: BP stages stop per frame at the first syndrome match (not the reference)
+        self.osd_order = int(osd_order)
+        if not 0 <= self.osd_order <= 65535:
+            raise ValueError(f"osd_order must be in [0, 65535], got {osd_order}")
         self._ctx = ctx
         self.last_counters = None
 
@@ -315,7 +319,7 @@ class Sandwich_BP_GNN_Evaluation_Model:
         thr = pauli_thresholds(0.0 if self.wt else float(p))
         cfg = _ffi.PipelineCfg(S, ni, fa, ct, gh, float(self.prior(p)), (C.c_float * 3)(*thr),
                                int(round(float(p))) if self.wt else 0, 1 if self.osd0 else 0,
-                               1 if self.skip_inactive else 0, 1 if self.early_stop else 0)
+                               1 if self.skip_inactive else 0, 1 if self.early_stop else 0, self.osd_order)
         return cfg, (ni, fa, ct, gh)
 
     def run(self, batch_size, p, noise=None, want_flags=True, want_diff=True, want_counters=False):
@@ -425,6 +429,7 @@ class BP_BSC_Model:
         self._logical = None
         self._osd_basis = None          # set by BP2_OSD_Model
         self._osd_pivot = None
+        self._osd_order = 0
         self.last_counters = None
 
     def llr_const(self, p):
@@ -454,11 +459,12 @@ class BP_BSC_Model:
                 raise ValueError(f"noise must have shape [{B},{self.n}], got {keep.shape}")
             nz = keep.t2()
         d = self.decoder
-        _ffi.call("fbgnn_bsc_pipeline_run", g.handle, lg.handle if lg is not None else None,
+        _ffi.call("fbgnn_bsc_pipeline_run_ex", g.handle, lg.handle if lg is not None else None,
                   CN_TYPES[d.cn_type], d.num_iter, d.normalization_factor, float(self.llr_const(p)),
                   float(np.float32(p)), self.seed, self.next_frame, B, nz, flags.ptr, counters,
                   self._osd_basis.handle if self._osd_basis is not None else None,
-                  self._osd_pivot.ctypes.data_as(C.POINTER(C.c_int32)) if self._osd_pivot is not None else None)
+                  self._osd_pivot.ctypes.data_as(C.POINTER(C.c_int32)) if self._osd_pivot is not None else None,
+                  self._osd_order)
         if noise is None:
             self.next_frame += B
         self.last_counters = np.array(list(counters), np.int64) if want_counters else None

@@ -16,6 +16,7 @@
  *   fbgnn_bsc_sample         <- BinarySymmetricChannel.call              channel/discrete_channel.py:385-396
  *   fbgnn_syndrome           <- int_mod_2(tf.matmul(H, noise))           feedback_gnn.py:308-309
  *   fbgnn_osd0_decode        <- OSD0_Decoder.call                        bp_osd.py:8-77
+ *   fbgnn_osd_decode         <- OSD0_Decoder.call + the OSD-CS sweep (Roffe et al. 2020; ldpc's osd_cs)
  *   fbgnn_gbp_create/_decode <- GNN_BP4.build / .call                    gnn.py:71-420
  *   fbgnn_pipeline_run       <- Sandwich_BP_GNN_Evaluation_Model.call    feedback_gnn.py:293-361
  *   fbgnn_bsc_pipeline_run   <- BP_BSC_Model.call                        feedback_gnn.py:207-229
@@ -227,6 +228,17 @@ int fbgnn_bp2_decode_ex(fbgnn_graph *graph, int32_t cn_type, int32_t num_iter, f
  * the syndrome reduced to the basis rows; e_hat uint8 (b, v) receives the error that satisfies it. */
 int fbgnn_osd0_decode(fbgnn_graph *basis, int64_t B, fbgnn_tensor2 llr, fbgnn_tensor2 synd,
                       fbgnn_tensor2 e_hat);
+/* Ordered-statistics decoding of order `order` with the combination sweep (OSD-CS; Roffe et al., "Decoding
+ * across the quantum LDPC code landscape", 2020; the `ldpc` package's osd_method="osd_cs").  Arguments as
+ * fbgnn_osd0_decode; order 0 is OSD-0, bit for bit.  With order lam > 0 the elimination of OSD-0 is followed,
+ * on the same reduced matrix, by a sweep over candidate sets T of the non-pivot columns c_0 < c_1 < ...
+ * (least reliable first): index 0 the empty set, 1 + i the single {c_i}, then the pairs {c_i, c_j},
+ * i < j < min(lam, n - rank), in lexicographic order.  T's solution is 1 on T and on pivot r the reduced
+ * syndrome bit XOR the columns of T in row r; the candidate of least (Hamming weight, index) is returned, so
+ * the result is the OSD-0 solution unless a candidate is strictly lighter.  order outside [0, 65535]:
+ * FBGNN_E_INVALID; a basis whose reduced matrix does not fit in shared memory: FBGNN_E_UNSUPPORTED. */
+int fbgnn_osd_decode(fbgnn_graph *basis, int32_t order, int64_t B, fbgnn_tensor2 llr, fbgnn_tensor2 synd,
+                     fbgnn_tensor2 e_hat);
 
 /* ---- feedback GNN --------------------------------------------------------------------- */
 /* Weights in Keras get_weights() order, host float32 pointers (copied); bias pointers may
@@ -311,6 +323,8 @@ typedef struct {
                                /*    (result-identical; the reference masks the scatter)     */
     int32_t early_stop;        /* 1: OPT-IN early stop inside every BP stage (see fbgnn_bp4_opts; NOT result-identical */
                                /*    to the reference in general -- a converged frame keeps its first converged state)  */
+    int32_t osd_order;         /* with osd0: 0 = OSD-0, lam in [1, 65535] = OSD-CS of order lam (fbgnn_osd_decode),     */
+                               /*    the same order on both sides (basis_x with osd_llrz, basis_z with osd_llrx)       */
 } fbgnn_pipeline_cfg;
 
 /* Sandwich_BP_GNN_Evaluation_Model.call on global frames [first_frame, first_frame+B).
@@ -347,6 +361,12 @@ int fbgnn_bsc_pipeline_run(fbgnn_graph *graph, fbgnn_graph *logical, int32_t cn_
                            int32_t num_iter, float factor, float llr_const, float p, uint64_t seed,
                            uint64_t first_frame, int64_t B, fbgnn_tensor2 noise, uint8_t *flags,
                            int64_t *counters, fbgnn_graph *osd_basis, const int32_t *osd_pivot);
+/* The same with OSD of order osd_order on the failed frames (0 = OSD-0, lam = OSD-CS; fbgnn_osd_decode). */
+int fbgnn_bsc_pipeline_run_ex(fbgnn_graph *graph, fbgnn_graph *logical, int32_t cn_type,
+                              int32_t num_iter, float factor, float llr_const, float p, uint64_t seed,
+                              uint64_t first_frame, int64_t B, fbgnn_tensor2 noise, uint8_t *flags,
+                              int64_t *counters, fbgnn_graph *osd_basis, const int32_t *osd_pivot,
+                              int32_t osd_order);
 
 /* ---- multi-GPU: the one collective of the path (SURVEY.md 8(e)) ------------------------- */
 /* Monte-Carlo frames shard across the GPUs of a box by global frame id; nothing but the counters is

@@ -1,0 +1,148 @@
+"""OSD-CS on a B200: kernel time per frame of fbgnn_osd_decode by order, and block errors of BP + OSD-{0, CS} on identical
+frames.  One run writes one JSON (default profiles/osd_bench.json):
+
+  kernel     fbgnn_osd_decode at B = 8192 for λ in {0, 1, 10, 30, 60}, on both sides of [[882,24]] and [[1270,28]]; the
+             reliabilities are the llr_x' / llr_z' (bp_osd.py:135-144) of a minsum BP4 decode (100 it., f = 0.8) at p = 0.10.
+             CUDA events around each launch, one warm-up launch, 7 timed launches: median, min and max.
+  ler        BP4(minsum, 100 it., f = 0.8) + OSD-{0, CS-10, CS-60} on [[882,24]], 300 000 frames at p = 0.10, the same seed
+             for all (examples/OSD.ipynb cell 2; published OSD-0: 111 / 300 000), and the n882.py Sandwich (nG = 5) without
+             OSD, with OSD-0 and with OSD-CS-10 at p = 0.10.
+
+Usage: python tools/osd_bench.py [--out FILE] [--frames 300000] [--kernel-only]
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.join(ROOT, "feedback-gnn_b200"))
+import numpy as np  # noqa: E402
+
+import fbgnn as F  # noqa: E402
+from fbgnn import _ffi  # noqa: E402
+
+ORDERS = (0, 1, 10, 30, 60)
+B_KERNEL = 8192
+REPS = 7
+
+
+def gpu_info():
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                       capture_output=True, text=True)
+    return q.stdout.strip() if q.returncode == 0 else f"nvidia-smi failed: {q.stderr.strip()}"
+
+
+def c882():
+    return F.create_QC_GHP_codes(63, F.create_cyclic_permuting_matrix(7, [27, 54, 0]), [0, 1, 6])
+
+
+def c1270():
+    return F.create_QC_GHP_codes(127, np.array([[0, -1, 51, 52, -1], [-1, 0, -1, 111, 20], [0, -1, 98, -1, 122],
+                                                [0, 80, -1, 119, -1], [-1, 0, 5, -1, 106]]), [0, 1, 7],
+                                 name="GHP_n1270_k28")
+
+
+def smem_bytes(n, R, lam):
+    """Dynamic shared memory of one k_osd CTA (launch_osd in csrc/fbgnn_pipeline.cu)."""
+    W, Rp = (n + 32) // 32, R | 1
+    npad = 1 << (n - 1).bit_length()
+    main = (max(npad * 8, W * Rp * 4) + 7) & ~7
+    u16 = 2 * (2 * n + R)
+    if lam == 0:
+        return main + u16 + 16
+    lp, RW = min(lam, max(n - R, 0)), (R + 31) // 32
+    return main + ((u16 + 15) & ~15) + (lp + 1) * RW * 4
+
+
+def kernel_times(code, ctx, seed):
+    """Per side: {order: {median_us_per_frame, min, max, ms_per_launch}}."""
+    n, B = code.N, B_KERNEL
+    nx, nz = F.Pauli(seed=seed).sample_device(B, n, F.pauli_thresholds(0.10))
+    gx, gz = _ffi.Graph(code.hx, ctx), _ffi.Graph(code.hz, ctx)
+    sx, sz = ctx.empty((B, gx.m), np.uint8), ctx.empty((B, gz.m), np.uint8)
+    _ffi.call("fbgnn_syndrome", gx.handle, B, nz.t2(), sx.T.t2())
+    _ffi.call("fbgnn_syndrome", gz.handle, B, nx.t2(), sz.T.t2())
+    dec = F.QLDPCBPDecoder(code, num_iter=100, normalization_factor=0.8, cn_type="minsum", stage_one=True)
+    Lx, Ly, Lz = (a.numpy().astype(np.float64) for a in dec((ctx.asarray(np.full((B, 3, n), np.log(27.0), np.float32)),
+                                                             sx.T, sz.T))[:3])
+    sp = lambda x: np.logaddexp(0.0, x)                                              # noqa: E731
+    llr_z = (sp(-Lx) - np.logaddexp(-Lz, -Ly)).astype(np.float32)                   # pairs with hx
+    llr_x = (sp(-Lz) - np.logaddexp(-Lx, -Ly)).astype(np.float32)                   # pairs with hz
+    sxh, szh = sx.numpy(), sz.numpy()
+    out = {}
+    for side, H, piv, llr, s in (("x", code.hx, code.pivot_hx, llr_z, sxh), ("z", code.hz, code.pivot_hz, llr_x, szh)):
+        basis = H[piv]
+        g = _ffi.Graph(basis, ctx)
+        R = basis.shape[0]
+        llr_d = ctx.asarray(llr, np.float32)
+        red_d = ctx.asarray(np.ascontiguousarray(s[:, piv].T), np.uint8)             # [rank, B]
+        e = ctx.empty((B, n), np.uint8)
+        res = {"rank": R, "n_minus_rank": n - R}
+        for lam in ORDERS:
+            run = lambda: _ffi.call("fbgnn_osd_decode", g.handle, lam, B, llr_d.t2(), red_d.t2(), e.t2())  # noqa: E731
+            run()
+            ctx.sync()
+            ms = []
+            for _ in range(REPS):
+                ctx.timer_start()
+                run()
+                ms.append(ctx.timer_stop())
+            ms = np.array(ms)
+            res[str(lam)] = {"us_per_frame_median": float(np.median(ms)) * 1e3 / B,
+                             "us_per_frame_min": float(ms.min()) * 1e3 / B, "us_per_frame_max": float(ms.max()) * 1e3 / B,
+                             "ms_per_launch": ms.tolist(), "smem_bytes_per_cta": smem_bytes(n, R, lam),
+                             "candidates": 1 + (0 if lam == 0 else (n - R) + min(lam, n - R) * (min(lam, n - R) - 1) // 2)}
+        out[side] = res
+    return out
+
+
+def count(model, frames, batch, p):
+    k, t0 = 0, time.perf_counter()
+    for _ in range(frames // batch):
+        k += int(model.run(batch, p, want_flags=False, want_diff=False, want_counters=True)["counters"][2])
+    return {"frames": frames, "block_errors": k, "seconds": time.perf_counter() - t0}
+
+
+def block_errors(frames, p=0.10, batch=50000, seed=70):
+    code = c882()
+    res = {}
+    dec = F.QLDPCBPDecoder(code, num_iter=100, normalization_factor=0.8, cn_type="minsum", stage_one=True)
+    for lam in (0, 10, 60):
+        model = F.BP4_OSD_Model(code, dec, F.OSD_Decoder(code.N, osd_order=lam), seed=seed)
+        model._inner.skip_inactive = True
+        res[f"bp4_osd_{'0' if lam == 0 else f'cs{lam}'}"] = count(model, frames, batch, p)
+    G = F.Feedback_GNN(code=code, num_msg_dims=20, num_hidden_units=40, num_mlp_layers=2, reduce_op="mean",
+                       activation="tanh", use_bias=True)
+    F.load_weights(G, os.path.join(F.WEIGHTS_DIR, "feedback_GNN_n882_k24_wt_4_60_iter_64_16_mixed.npy"))
+    d1 = F.QLDPCBPDecoder(code=code, num_iter=64, normalization_factor=1.0, cn_type="boxplus-phi", stage_one=True)
+    d2 = F.QLDPCBPDecoder(code=code, num_iter=16, normalization_factor=1.0, cn_type="boxplus-phi", stage_one=True)
+    for name, kw in (("sandwich_nG5", {}), ("sandwich_nG5_osd0", dict(osd0=True)),
+                     ("sandwich_nG5_osd_cs10", dict(osd0=True, osd_order=10))):
+        model = F.Sandwich_BP_GNN_Evaluation_Model(code, [d1] + [d2] * 5, [G] * 5, num_layers=6, skip_inactive=True,
+                                                   seed=seed, **kw)
+        res[name] = count(model, frames, batch, p)
+    return res
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "osd_bench.json"))
+    ap.add_argument("--frames", type=int, default=300000)
+    ap.add_argument("--kernel-only", action="store_true")
+    args = ap.parse_args()
+    ctx = F.default_context()
+    res = {"device": ctx.name, "nvidia_smi": gpu_info(), "math": ctx.get_math(), "B": B_KERNEL, "reps": REPS,
+           "kernel": {"c882": kernel_times(c882(), ctx, 1), "c1270": kernel_times(c1270(), ctx, 2)}}
+    if not args.kernel_only:
+        res["block_errors_p010"] = block_errors(args.frames)
+    os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+    with open(args.out, "w") as f:
+        json.dump(res, f, indent=1)
+    print(json.dumps(res)[:4000])
+
+
+if __name__ == "__main__":
+    main()
