@@ -2108,22 +2108,61 @@ __device__ __forceinline__ void osd_pair(int64_t q, int lp, int &i, int &j) {
     j = (int)(i + 1 + (q - start(i)));
 }
 
-// smem: max(npad * 8, W * Rp * 4) bytes shared by the sort keys and the matrix; u16 order[n], inv[n], piv[R];
-// with order > 0, at cv_off: u32 cv[lp][RW] (the first lp non-pivot columns over the rows) and sv[RW] (s')
-static __global__ void __launch_bounds__(256) k_osd(const OsdArgs a) {
-    extern __shared__ unsigned long long osd_smem[];
-    const SideDev &S = a.S;
-    const int n = S.n, R = S.m, T = blockDim.x, tid = threadIdx.x;
-    const int W = (n + 1 + 31) / 32, Rp = R | 1;                 // odd stride: no bank conflicts across words
-    const int64_t b = a.frame_list ? a.frame_list[blockIdx.x] : blockIdx.x;
-    unsigned long long *keys = osd_smem;
-    uint32_t *M = (uint32_t *)osd_smem;
-    const size_t main_bytes = ((size_t)a.npad * 8 > (size_t)W * Rp * 4) ? (size_t)a.npad * 8 : (size_t)W * Rp * 4;
-    uint16_t *order = (uint16_t *)((uint8_t *)osd_smem + ((main_bytes + 7) & ~(size_t)7));
-    uint16_t *inv = order + n, *piv = inv + n;
-    __shared__ int cur_p;
+// one warp: the first column < n set in row `row` of the word-major bit matrix M (row stride Rp), 0 if none; the same
+// value in every lane.  wn = n / 32; last_mask keeps the columns < n of word wn.
+__device__ __forceinline__ int osd_pivot(const uint32_t *M, int Rp, int row, int W, int wn, uint32_t last_mask, int lane) {
+    int p = 0, found = 0;
+    for (int w0 = 0; w0 < W && !found; w0 += 32) {
+        const int w = w0 + lane;
+        uint32_t word = w < W ? M[w * Rp + row] : 0u;
+        if (w == wn) word &= last_mask;
+        if (w > wn) word = 0u;
+        const uint32_t vote = __ballot_sync(0xffffffffu, word != 0u);
+        if (vote) {
+            const int l = __ffs(vote) - 1;
+            const uint32_t wsel = __shfl_sync(0xffffffffu, word, l);
+            p = (w0 + l) * 32 + (__ffs(wsel) - 1);
+            found = 1;
+        }
+    }
+    return p;
+}
 
-    // 1. stable ascending sort of the reliabilities (bitonic network on (key, index) pairs)
+// OSD-CS step 4c, for every thread of the CTA: fold the pairs of the first lp non-pivot columns (bit vectors cv[lp][RW]
+// and s' in sv[RW]) into this thread's least (weight << 32 | index), then take the CTA's least into *best (set to ~0
+// beforehand and read after a __syncthreads).  N is the number of non-pivot columns.
+__device__ __forceinline__ void osd_cs_best(unsigned long long mine, const uint32_t *cv, const uint32_t *sv, int RW, int lp,
+                                            int N, unsigned long long *best) {
+    const int64_t P = (int64_t)lp * (lp - 1) / 2;
+    for (int64_t q = threadIdx.x; q < P; q += blockDim.x) {
+        int i, j;
+        osd_pair(q, lp, i, j);
+        int w = 2;
+        for (int k = 0; k < RW; k++) w += __popc(sv[k] ^ cv[i * RW + k] ^ cv[j * RW + k]);
+        mine = min(mine, ((unsigned long long)w << 32) | (uint32_t)(1 + N + q));
+    }
+    for (int o = 16; o > 0; o >>= 1) mine = min(mine, __shfl_xor_sync(0xffffffffu, mine, o));
+    if ((threadIdx.x & 31) == 0) atomicMin(best, mine);
+}
+
+// candidate index -> its columns t0 / t1 (-1: none); np lists the non-pivot columns in increasing position
+__device__ __forceinline__ void osd_cs_columns(uint32_t idx, int N, int lp, const uint16_t *np, int &t0, int &t1) {
+    if (idx >= 1 && idx <= (uint32_t)N) t0 = np[idx - 1];
+    else if (idx > (uint32_t)N) {
+        int i, j;
+        osd_pair((int64_t)idx - 1 - N, lp, i, j);
+        t0 = np[i]; t1 = np[j];
+    }
+}
+
+// Steps of k_osd that the cluster form (k_osd_cluster, fbgnn_osd_cluster.cuh) runs too.  Each is called by every thread
+// of the CTA and ends with the CTA's writes visible to all its threads.
+
+// 1. stable ascending sort of sign * llr(b, .) (bitonic network on (key, index) pairs): order[j] = the column at
+//    position j, inv[v] = the position of column v
+__device__ __forceinline__ void osd_sort(const OsdArgs &a, int64_t b, unsigned long long *keys, uint16_t *order,
+                                         uint16_t *inv) {
+    const int n = a.S.n, T = blockDim.x, tid = threadIdx.x;
     for (int i = tid; i < a.npad; i += T)
         keys[i] = i < n ? osd_key(a.sign * a.llr(b, i), i) : ~0ull;
     __syncthreads();
@@ -2146,39 +2185,104 @@ static __global__ void __launch_bounds__(256) k_osd(const OsdArgs a) {
         inv[v] = (uint16_t)j;
     }
     __syncthreads();
+}
 
-    // 2. permuted [H | s] as a bit matrix, one thread per row
+// 2. basis rows r0 .. r0 + nr - 1 of the permuted [H | s] as rows 0 .. nr - 1 of the bit matrix M (word-major, row
+//    stride Rp, W words), one thread per row
+__device__ __forceinline__ void osd_build_rows(const OsdArgs &a, int64_t b, uint32_t *M, int Rp, const uint16_t *inv,
+                                               int r0, int nr) {
+    const SideDev &S = a.S;
+    const int n = S.n, W = (n + 1 + 31) / 32, T = blockDim.x, tid = threadIdx.x;
     for (int i = tid; i < W * Rp; i += T) M[i] = 0u;
     __syncthreads();
-    for (int r = tid; r < R; r += T) {
+    for (int i = tid; i < nr; i += T) {
+        const int r = r0 + i;
         for (int k = S.cn_ptr[r]; k < S.cn_ptr[r + 1]; k++) {
             const int j = inv[S.cn_vn[k]];
-            M[(j >> 5) * Rp + r] ^= 1u << (j & 31);
+            M[(j >> 5) * Rp + i] ^= 1u << (j & 31);
         }
         const int sr = a.synd_row ? a.synd_row[r] : r;
-        if (a.synd(sr, b)) M[(n >> 5) * Rp + r] ^= 1u << (n & 31);
+        if (a.synd(sr, b)) M[(n >> 5) * Rp + i] ^= 1u << (n & 31);
     }
     __syncthreads();
+}
+
+// 4a. the non-pivot columns in increasing position into np[0 .. *num - 1]; np (n entries) is overwritten
+__device__ __forceinline__ void osd_cs_list(uint16_t *np, const uint16_t *piv, int n, int R, int *num) {
+    const int T = blockDim.x, tid = threadIdx.x, lane = tid & 31;
+    for (int j = tid; j < n; j += T) np[j] = 1;
+    __syncthreads();
+    for (int r = tid; r < R; r += T) np[piv[r]] = 0;
+    __syncthreads();
+    if (tid < 32) {
+        int cnt = 0;
+        for (int j0 = 0; j0 < n; j0 += 32) {                       // list position <= column: reads stay ahead of writes
+            const int j = j0 + lane;
+            const bool np_col = j < n && np[j];
+            const uint32_t vote = __ballot_sync(0xffffffffu, np_col);
+            if (np_col) np[cnt + __popc(vote & ((1u << lane) - 1u))] = (uint16_t)j;
+            cnt += __popc(vote);
+        }
+        if (lane == 0) *num = cnt;
+    }
+    __syncthreads();
+}
+
+// 5. the solution on the pivot columns of bit-matrix rows 0 .. nr - 1 (their pivots in piv[0 .. nr - 1]) and, with
+//    with_t, on the columns t0 / t1 of the winning candidate, mapped back through the permutation.  The frame's
+//    outputs must have been cleared before.
+__device__ __forceinline__ void osd_write_solution(const OsdArgs &a, int64_t b, const uint32_t *M, int Rp,
+                                                   const uint16_t *order, const uint16_t *piv, int nr, int t0, int t1,
+                                                   bool with_t) {
+    const int n = a.S.n, wn = n >> 5, T = blockDim.x, tid = threadIdx.x;
+    for (int r = tid; r < nr; r += T) {
+        int sol = (M[wn * Rp + r] >> (n & 31)) & 1u;
+        if (t0 >= 0) sol ^= (M[(t0 >> 5) * Rp + r] >> (t0 & 31)) & 1u;
+        if (t1 >= 0) sol ^= (M[(t1 >> 5) * Rp + r] >> (t1 & 31)) & 1u;
+        const int v = order[piv[r]];
+        if (sol) {
+            if (a.e_hat.ptr) a.e_hat(b, v) = 1;
+            if (a.vbits) a.vbits[b * n + v] |= (uint8_t)(1u << a.vbit);
+        }
+    }
+    if (with_t && tid == 0) {
+        for (int e = 0; e < 2; e++) {
+            const int c = e ? t1 : t0;
+            if (c < 0) continue;
+            const int v = order[c];
+            if (a.e_hat.ptr) a.e_hat(b, v) = 1;
+            if (a.vbits) a.vbits[b * n + v] |= (uint8_t)(1u << a.vbit);
+        }
+    }
+}
+
+// smem: max(npad * 8, W * Rp * 4) bytes shared by the sort keys and the matrix; u16 order[n], inv[n], piv[R];
+// with order > 0, at cv_off: u32 cv[lp][RW] (the first lp non-pivot columns over the rows) and sv[RW] (s')
+static __global__ void __launch_bounds__(256) k_osd(const OsdArgs a) {
+    extern __shared__ unsigned long long osd_smem[];
+    const SideDev &S = a.S;
+    const int n = S.n, R = S.m, T = blockDim.x, tid = threadIdx.x;
+    const int W = (n + 1 + 31) / 32, Rp = R | 1;                 // odd stride: no bank conflicts across words
+    const int64_t b = a.frame_list ? a.frame_list[blockIdx.x] : blockIdx.x;
+    unsigned long long *keys = osd_smem;
+    uint32_t *M = (uint32_t *)osd_smem;
+    const size_t main_bytes = ((size_t)a.npad * 8 > (size_t)W * Rp * 4) ? (size_t)a.npad * 8 : (size_t)W * Rp * 4;
+    uint16_t *order = (uint16_t *)((uint8_t *)osd_smem + ((main_bytes + 7) & ~(size_t)7));
+    uint16_t *inv = order + n, *piv = inv + n;
+    __shared__ int cur_p;
+
+    // 1. stable ascending sort of the reliabilities
+    osd_sort(a, b, keys, order, inv);
+
+    // 2. permuted [H | s] as a bit matrix, one thread per row
+    osd_build_rows(a, b, M, Rp, inv, 0, R);
 
     // 3. row-wise elimination
     const int wn = n >> 5;
     const uint32_t last_mask = (n & 31) ? ((1u << (n & 31)) - 1u) : 0u;   // columns < n inside word wn
     for (int r = 0; r < R; r++) {
         if (tid < 32) {
-            int p = 0, found = 0;
-            for (int w0 = 0; w0 < W && !found; w0 += 32) {
-                const int w = w0 + tid;
-                uint32_t word = w < W ? M[w * Rp + r] : 0u;
-                if (w == wn) word &= last_mask;
-                if (w > wn) word = 0u;
-                const uint32_t vote = __ballot_sync(0xffffffffu, word != 0u);
-                if (vote) {
-                    const int lane = __ffs(vote) - 1;
-                    const uint32_t wsel = __shfl_sync(0xffffffffu, word, lane);
-                    p = (w0 + lane) * 32 + (__ffs(wsel) - 1);
-                    found = 1;
-                }
-            }
+            const int p = osd_pivot(M, Rp, r, W, wn, last_mask, tid);
             if (tid == 0) { cur_p = p; piv[r] = (uint16_t)p; }
         }
         __syncthreads();
@@ -2200,23 +2304,9 @@ static __global__ void __launch_bounds__(256) k_osd(const OsdArgs a) {
         const int RW = (R + 31) / 32, lp = min(a.order, max(n - R, 0));
         const int lane = tid & 31, warp = tid >> 5, nw = T >> 5;
         uint32_t *cv = (uint32_t *)((uint8_t *)osd_smem + a.cv_off), *sv = cv + (size_t)lp * RW;
-        // 4a. the non-pivot columns in increasing position, listed in inv (free since step 2); s' as a bit vector
-        for (int j = tid; j < n; j += T) inv[j] = 1;
+        // 4a. the non-pivot columns listed in inv (free since step 2); s' as a bit vector
         if (tid == 0) best = ~0ull;
-        __syncthreads();
-        for (int r = tid; r < R; r += T) inv[piv[r]] = 0;
-        __syncthreads();
-        if (warp == 0) {
-            int cnt = 0;
-            for (int j0 = 0; j0 < n; j0 += 32) {                   // list position <= column: reads stay ahead of writes
-                const int j = j0 + lane;
-                const bool np_col = j < n && inv[j];
-                const uint32_t vote = __ballot_sync(0xffffffffu, np_col);
-                if (np_col) inv[cnt + __popc(vote & ((1u << lane) - 1u))] = (uint16_t)j;
-                cnt += __popc(vote);
-            }
-            if (lane == 0) num_np = cnt;
-        }
+        osd_cs_list(inv, piv, n, R, &num_np);
         for (int k = warp; k < RW; k += nw) {
             const int r = k * 32 + lane;
             const uint32_t v = __ballot_sync(0xffffffffu, r < R && ((M[wn * Rp + r] >> (n & 31)) & 1u));
@@ -2245,49 +2335,16 @@ static __global__ void __launch_bounds__(256) k_osd(const OsdArgs a) {
         }
         __syncthreads();
         // 4c. pairs of the first lp columns, one thread per pair
-        const int64_t P = (int64_t)lp * (lp - 1) / 2;
-        for (int64_t q = tid; q < P; q += T) {
-            int i, j;
-            osd_pair(q, lp, i, j);
-            int w = 2;
-            for (int k = 0; k < RW; k++) w += __popc(sv[k] ^ cv[i * RW + k] ^ cv[j * RW + k]);
-            mine = min(mine, ((unsigned long long)w << 32) | (uint32_t)(1 + N + q));
-        }
-        for (int o = 16; o > 0; o >>= 1) mine = min(mine, __shfl_xor_sync(0xffffffffu, mine, o));
-        if (lane == 0) atomicMin(&best, mine);
+        osd_cs_best(mine, cv, sv, RW, lp, N, &best);
         __syncthreads();
-        const uint32_t idx = (uint32_t)best;
-        if (idx >= 1 && idx <= (uint32_t)N) t0 = inv[idx - 1];
-        else if (idx > (uint32_t)N) {
-            int i, j;
-            osd_pair((int64_t)idx - 1 - N, lp, i, j);
-            t0 = inv[i]; t1 = inv[j];
-        }
+        osd_cs_columns((uint32_t)best, N, lp, inv, t0, t1);
     }
 
     // 5. the solution on the pivot columns and on T, mapped back through the permutation
     if (a.e_hat.ptr) for (int v = tid; v < n; v += T) a.e_hat(b, v) = 0;
     if (a.vbits) for (int v = tid; v < n; v += T) a.vbits[b * n + v] &= (uint8_t)~(1u << a.vbit);
     __syncthreads();
-    for (int r = tid; r < R; r += T) {
-        int sol = (M[wn * Rp + r] >> (n & 31)) & 1u;
-        if (t0 >= 0) sol ^= (M[(t0 >> 5) * Rp + r] >> (t0 & 31)) & 1u;
-        if (t1 >= 0) sol ^= (M[(t1 >> 5) * Rp + r] >> (t1 & 31)) & 1u;
-        const int v = order[piv[r]];
-        if (sol) {
-            if (a.e_hat.ptr) a.e_hat(b, v) = 1;
-            if (a.vbits) a.vbits[b * n + v] |= (uint8_t)(1u << a.vbit);
-        }
-    }
-    if (tid == 0) {
-        for (int e = 0; e < 2; e++) {
-            const int c = e ? t1 : t0;
-            if (c < 0) continue;
-            const int v = order[c];
-            if (a.e_hat.ptr) a.e_hat(b, v) = 1;
-            if (a.vbits) a.vbits[b * n + v] |= (uint8_t)(1u << a.vbit);
-        }
-    }
+    osd_write_solution(a, b, M, Rp, order, piv, R, t0, t1, true);
 }
 
 // reliabilities handed to OSD-0 by BP4_OSD_Model (bp_osd.py:135-144), for the listed frames:

@@ -1,27 +1,88 @@
 // fbgnn_pipeline.cu -- the fused Monte-Carlo pipelines (multi-launch orchestration) and OSD.
 #include "fbgnn_internal.h"
+#include "fbgnn_osd_cluster.cuh"
 
 // ------------------------------------------------------------------ OSD -----------------
+// Dynamic shared memory of one OSD CTA that holds `rows` basis rows; with `cluster`, the layout of k_osd_cluster (its
+// slots after the u16 arrays, and csum[n] after cv / sv).  Sets a.cv_off (order > 0) and *slot_off.
+static size_t osd_smem(OsdArgs &a, int rows, bool cluster, int *slot_off) {
+    const int n = a.S.n, R = a.S.m, W = (n + 1 + 31) / 32, Rp = rows | 1;
+    const size_t main_bytes = std::max<size_t>((size_t)a.npad * 8, (size_t)W * Rp * 4);
+    const size_t u16_bytes = sizeof(uint16_t) * (2 * (size_t)n + R);
+    size_t smem = ((main_bytes + 7) & ~(size_t)7) + u16_bytes + 16;
+    size_t cs_base = ((main_bytes + 7) & ~(size_t)7) + ((u16_bytes + 15) & ~(size_t)15);
+    if (cluster) {              // slot[2][W + 1], row[W + 1], svl[rows / 32]
+        *slot_off = (int)cs_base;
+        smem = cs_base + sizeof(uint32_t) * (3 * ((size_t)W + 1) + (size_t)rows / 32);
+        cs_base = (smem + 15) & ~(size_t)15;
+    }
+    if (a.order > 0) {          // OSD-CS: the first lp non-pivot columns and s' as ceil(R/32)-word bit vectors
+        const size_t lp = (size_t)std::min(a.order, std::max(n - R, 0)), RW = ((size_t)R + 31) / 32;
+        a.cv_off = (int)cs_base;
+        smem = cs_base + (lp + 1) * RW * 4 + (cluster ? sizeof(int) * (size_t)n : 0);
+    }
+    return smem;
+}
+
 int launch_osd(fbgnn_ctx *ctx, OsdArgs &a, int order, int64_t grid) {
     if (grid <= 0) return 0;
-    const int n = a.S.n, R = a.S.m, W = (n + 1 + 31) / 32, Rp = R | 1;
+    const int n = a.S.n, R = a.S.m;
     int npad = 1;
     while (npad < n) npad <<= 1;
     a.npad = npad;
     a.order = order;
-    const size_t main_bytes = std::max<size_t>((size_t)npad * 8, (size_t)W * Rp * 4);
-    const size_t u16_bytes = sizeof(uint16_t) * (2 * (size_t)n + R);
-    size_t smem = ((main_bytes + 7) & ~(size_t)7) + u16_bytes + 16;
-    if (order > 0) {            // OSD-CS: the first lp non-pivot columns and s' as ceil(R/32)-word bit vectors
-        const size_t lp = (size_t)std::min(order, std::max(n - R, 0)), RW = ((size_t)R + 31) / 32;
-        a.cv_off = (int)(((main_bytes + 7) & ~(size_t)7) + ((u16_bytes + 15) & ~(size_t)15));
-        smem = (size_t)a.cv_off + (lp + 1) * RW * 4;
+    const char *what = order > 0 ? "OSD-CS" : "OSD-0";
+    int unused;
+    const size_t smem = osd_smem(a, R, false, &unused);
+    // FBGNN_OSD_CLUSTER=<C> (2, 4 or 8; read at every launch) runs the cluster kernel where one CTA would do, so that
+    // small codes test it against k_osd.
+    int force = 0;
+    if (const char *e = getenv("FBGNN_OSD_CLUSTER")) {
+        force = atoi(e);
+        REQUIRE(force == 2 || force == 4 || force == 8, "FBGNN_OSD_CLUSTER=%s: expected 2, 4 or 8", e);
     }
-    if (int rc = set_smem(k_osd, smem, ctx, order > 0 ? "OSD-CS" : "OSD-0")) return rc;
-    k_osd<<<(unsigned)grid, 256, smem, ctx->stream>>>(a);
-    CK(cudaGetLastError());
-    ctx->launches++;
-    return 0;
+    if (!force && smem <= ctx->smem_optin) {
+        if (int rc = set_smem(k_osd, smem, ctx, what)) return rc;
+        k_osd<<<(unsigned)grid, 256, smem, ctx->stream>>>(a);
+        CK(cudaGetLastError());
+        ctx->launches++;
+        return 0;
+    }
+    // The matrix exceeds one CTA: the smallest cluster of 2 / 4 / 8 CTAs whose per-CTA rows fit (fbgnn_osd_cluster.cuh).
+    // Every CTA gets the largest per-rank footprint: its share of the rows plus, for rank 0, the OSD-CS vectors.
+    size_t smem_cl = 0;
+    for (int C = force ? force : 2; C <= OSD_CL_MAX; C *= 2) {
+        OsdCluster P{};
+        P.C = C;
+        P.rs = ((R + 31) / 32 + C - 1) / C * 32;
+        smem_cl = osd_smem(a, P.rs, true, &P.slot_off);
+        if (smem_cl > ctx->smem_optin) {
+            if (force) break;
+            continue;
+        }
+        CK(cudaFuncSetAttribute(k_osd_cluster, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_cl));
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = dim3((unsigned)(grid * C), 1, 1);
+        cfg.blockDim = dim3(256, 1, 1);
+        cfg.dynamicSmemBytes = smem_cl;
+        cfg.stream = ctx->stream;
+        cudaLaunchAttribute attr[1];
+        attr[0].id = cudaLaunchAttributeClusterDimension;
+        attr[0].val.clusterDim.x = (unsigned)C; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+        cfg.attrs = attr; cfg.numAttrs = 1;
+        int clusters = 0;
+        CK(cudaOccupancyMaxActiveClusters(&clusters, k_osd_cluster, &cfg));
+        if (clusters <= 0) {
+            if (force) break;
+            continue;
+        }
+        CK(cudaLaunchKernelEx(&cfg, k_osd_cluster, a, P));
+        ctx->launches++;
+        return 0;
+    }
+    return fail(FBGNN_E_UNSUPPORTED, "%s needs %zu bytes of shared memory per frame in one CTA and %zu per CTA in a "
+                "cluster of %d; the device offers %zu per CTA", what, smem, smem_cl, force ? force : OSD_CL_MAX,
+                ctx->smem_optin);
 }
 
 // OSD-CS candidate indices are 32-bit: 1 + N + lp (lp - 1) / 2 < 2^32 for lp <= 65535

@@ -15,6 +15,11 @@ OSD-0 solution; the lightest solution (Hamming weight, ties to the earlier candi
 
 Ties between equal reliabilities are broken by qubit index (the reference's ``tf.argsort`` leaves
 them to the backend).
+
+A frame's reduced matrix sits in the shared memory of one CTA (``k_osd``).  Where it does not fit, as for the
+[[1922,50]] hypergraph-product code, a thread-block cluster of 2, 4 or 8 CTAs splits it by rows (``k_osd_cluster``,
+the same result bit for bit).  A basis beyond a cluster of 8 (about 1.8 MB, e.g. [[7688,50]]) raises ``FbgnnError``
+with ``FBGNN_E_UNSUPPORTED`` (-3).
 """
 import numpy as np
 

@@ -236,7 +236,9 @@ int fbgnn_osd0_decode(fbgnn_graph *basis, int64_t B, fbgnn_tensor2 llr, fbgnn_te
  * i < j < min(lam, n - rank), in lexicographic order.  T's solution is 1 on T and on pivot r the reduced
  * syndrome bit XOR the columns of T in row r; the candidate of least (Hamming weight, index) is returned, so
  * the result is the OSD-0 solution unless a candidate is strictly lighter.  order outside [0, 65535]:
- * FBGNN_E_INVALID; a basis whose reduced matrix does not fit in shared memory: FBGNN_E_UNSUPPORTED. */
+ * FBGNN_E_INVALID.  A frame's reduced matrix lives in the shared memory of one CTA or, when it does not fit there,
+ * is split by rows over a thread-block cluster of 2, 4 or 8 CTAs (same result, bit for bit); a basis that does
+ * not fit a cluster of 8 either returns FBGNN_E_UNSUPPORTED, with the bytes it needs in the message. */
 int fbgnn_osd_decode(fbgnn_graph *basis, int32_t order, int64_t B, fbgnn_tensor2 llr, fbgnn_tensor2 synd,
                      fbgnn_tensor2 e_hat);
 
