@@ -393,6 +393,74 @@ FB_HD float fb_sfu_atanhf(float x) {
     return FB_MUL(0.5f, FB_SUB(fb_sfu_logf(FB_ADD(1.0f, x)), fb_sfu_logf(FB_SUB(1.0f, x))));
 }
 
+#if defined(__CUDACC__) && (!defined(__CUDA_ARCH__) || __CUDA_ARCH__ >= 1000)
+/* ---- paired SFU arithmetic (device only, sm_100 and later) -----------------------------------------------------------------------
+ * float2 forms of the SFU functions above for sm_100's packed FP32 instructions fma.rn.f32x2 / add.rn.f32x2 /
+ * mul.rn.f32x2 (SASS FFMA2 / FADD2 / FMUL2): two float32 operations in one issue slot, each lane rounded to nearest
+ * exactly as the scalar __fmaf_rn / __fadd_rn / __fmul_rn round it, without flushing subnormals.  Each lane performs
+ * the scalar function's IEEE operations in the same order with the same constants; the MUFU, the exponent splices,
+ * min / max and the compares stay scalar per lane.  The scalar functions remain the specification (the CPU oracle
+ * evaluates those), and tests/test_gpu_sfu_pairs.py holds every paired form to its scalar form bit for bit.
+ * a - b is formed as a + (-b), which IEEE-754 defines it to be (signed zeros included). */
+__device__ __forceinline__ float2 fb2(float a, float b) { return make_float2(a, b); }
+__device__ __forceinline__ float2 fb2s(float a) { return make_float2(a, a); }
+__device__ __forceinline__ float2 fb2_neg(float2 a) { return make_float2(-a.x, -a.y); }
+#define FB_FMA2(a, b, c) __ffma2_rn((a), (b), (c))
+#define FB_ADD2(a, b)    __fadd2_rn((a), (b))
+#define FB_SUB2(a, b)    __fadd2_rn((a), fb2_neg(b))
+#define FB_MUL2(a, b)    __fmul2_rn((a), (b))
+
+__device__ __forceinline__ float2 fb_sfu_exp2s2(float2 x, float c) {
+    const float2 t = FB_FMA2(x, fb2s(c), fb2s(12582911.0f));
+    const float2 fn = FB_SUB2(t, fb2s(12582912.0f));
+    const float2 u = FB_FMA2(x, fb2s(c), fb2_neg(fn));
+    const float yx = fb_mufu_ex2(u.x), yy = fb_mufu_ex2(u.y);
+    return fb2(FB_I2F(FB_F2I(yx) + (int32_t)((uint32_t)FB_F2I(t.x) << 23)),
+               FB_I2F(FB_F2I(yy) + (int32_t)((uint32_t)FB_F2I(t.y) << 23)));
+}
+__device__ __forceinline__ float2 fb_sfu_logaddexp_open2(float2 mx, float2 d) {
+    const float2 s = FB_ADD2(fb2s(1.0f), fb_sfu_exp2s2(d, FB_LOG2E));
+    return FB_FMA2(fb2(fb_mufu_lg2(s.x), fb_mufu_lg2(s.y)), fb2s(FB_LN2), mx);
+}
+__device__ __forceinline__ float2 fb_sfu_softplusf2(float2 x) {
+    const float2 ax = fb2(FB_FMIN(FB_I2F(FB_F2I(x.x) & 0x7fffffff), 86.0f), FB_FMIN(FB_I2F(FB_F2I(x.y) & 0x7fffffff), 86.0f));
+    const float2 e = fb_sfu_exp2s2(ax, -FB_LOG2E);
+    const float2 s = FB_ADD2(fb2s(1.0f), e);
+    float2 r = FB_FMA2(fb2(fb_mufu_lg2(s.x), fb_mufu_lg2(s.y)), fb2s(FB_LN2), fb2(FB_FMAX(x.x, 0.0f), FB_FMAX(x.y, 0.0f)));
+    r.x = (x.x < -FB_SOFTPLUS_THR) ? e.x : r.x;
+    r.y = (x.y < -FB_SOFTPLUS_THR) ? e.y : r.y;
+    return fb2((x.x > FB_SOFTPLUS_THR) ? x.x : r.x, (x.y > FB_SOFTPLUS_THR) ? x.y : r.y);
+}
+__device__ __forceinline__ float2 fb_sfu_vn_corr2(float2 l1, float2 ly) {
+    float2 d = FB_SUB2(ly, l1);
+    d = fb2(FB_I2F(FB_F2I(d.x) | (int32_t)0x80000000), FB_I2F(FB_F2I(d.y) | (int32_t)0x80000000));
+    const float2 f = fb_sfu_logaddexp_open2(fb2s(0.0f), fb2(FB_FMAX(d.x, -17.5f), FB_FMAX(d.y, -17.5f)));
+    return fb2((d.x < -17.5f) ? 0.0f : f.x, (d.y < -17.5f) ? 0.0f : f.y);
+}
+__device__ __forceinline__ float2 fb_sfu_vn_msg2(float2 num, float2 a, float2 u, float2 corr) {
+    return FB_SUB2(num, FB_ADD2(FB_SUB2(a, u), corr));
+}
+__device__ __forceinline__ float2 fb_sfu_phi_open2(float2 x) {
+    const float2 t = fb_sfu_exp2s2(x, -FB_LOG2E);
+    const float2 sa = FB_ADD2(fb2s(1.0f), t), sb = FB_SUB2(fb2s(1.0f), t);
+    const float2 la = fb2(fb_mufu_lg2(sa.x), fb_mufu_lg2(sa.y));
+    const float2 lb = fb2(fb_mufu_lg2(FB_FMAX(sb.x, 1.1920928955078125e-7f)), fb_mufu_lg2(FB_FMAX(sb.y, 1.1920928955078125e-7f)));
+#if FB_SFU_PHI_STABLE
+    return FB_MUL2(FB_SUB2(la, lb), fb2s(FB_LN2));
+#else
+    return FB_SUB2(FB_FMA2(la, fb2s(FB_LN2), x), FB_FMA2(lb, fb2s(FB_LN2), x));
+#endif
+}
+__device__ __forceinline__ float2 fb_sfu_tanhf2(float2 x) {
+    const float2 ax = fb2(FB_FMIN(FB_I2F(FB_F2I(x.x) & 0x7fffffff), 10.0f), FB_FMIN(FB_I2F(FB_F2I(x.y) & 0x7fffffff), 10.0f));
+    const float2 t = fb_sfu_exp2s2(ax, -2.0f * FB_LOG2E);
+    const float2 q = FB_ADD2(fb2s(1.0f), t);
+    const float2 r = FB_MUL2(FB_SUB2(fb2s(1.0f), t), fb2(fb_mufu_rcp(q.x), fb_mufu_rcp(q.y)));
+    return fb2(FB_I2F(FB_F2I(r.x) | (FB_F2I(x.x) & (int32_t)0x80000000)),
+               FB_I2F(FB_F2I(r.y) | (FB_F2I(x.y) & (int32_t)0x80000000)));
+}
+#endif
+
 #if !defined(__CUDACC__)
 /* ---- host-side arithmetic selection (the CPU oracle): 0 = exact (default), 1 = SFU ------------ */
 static int fb_math_mode = 0;

@@ -513,9 +513,13 @@ extern "C" int fbgnn_math_probe(fbgnn_ctx *ctx, const char *fn, const float *x, 
     REQUIRE(ctx && fn && x && y && n >= 0, "bad argument");
     static const char *names[] = {"exp", "log", "log1p", "softplus", "phi4", "phi2", "tanh", "atanh", "mufu_ex2",
                                   "mufu_lg2", "sfu_exp", "sfu_log", "sfu_softplus", "sfu_phi4", "sfu_phi2", "mufu_rcp",
-                                  "sfu_tanh", "sfu_atanh"};
+                                  "sfu_tanh", "sfu_atanh", nullptr, nullptr,
+                                  // 20..24: scalar SFU building blocks; 25..31: their paired (float2) forms
+                                  "sfu_exp2s", "sfu_logaddexp_open", "sfu_vn_corr", "sfu_vn_msg", "sfu_phi_open",
+                                  "sfu2_exp2s", "sfu2_logaddexp_open", "sfu2_vn_corr", "sfu2_vn_msg", "sfu2_phi_open",
+                                  "sfu2_softplus", "sfu2_tanh"};
     int id = -1;
-    for (int i = 0; i < 18; i++) if (!std::strcmp(fn, names[i])) id = i;
+    for (int i = 0; i < (int)(sizeof(names) / sizeof(names[0])); i++) if (names[i] && !std::strcmp(fn, names[i])) id = i;
     REQUIRE(id >= 0, "unknown probe function '%s'", fn);
     if (set_device(ctx)) return FBGNN_E_CUDA;
     if (n == 0) return 0;

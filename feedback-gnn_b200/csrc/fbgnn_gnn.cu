@@ -61,6 +61,13 @@ extern "C" int fbgnn_gnn_create(fbgnn_ctx *ctx, int32_t H, int32_t M, int32_t ac
         tile(GnnW::W2Z, 40, 32, [&](int k, int nn) { return nn < 20 ? W2z[k * 20 + nn] * inv : 0.0f; });
         tile(GnnW::W3AB, 40, 48, [&](int k, int nn) { return nn < 40 ? W3[k * 40 + nn] : 0.0f; });
         std::memcpy(&tv[GnnW::SCALAR], w.data(), sizeof(float) * w.size());
+        // first-layer rows of hidden units j, j+1 interleaved (k_gnn_tc's edge phase evaluates them as a pair)
+        typedef GnnLayout<40, 20> L;
+        for (int j = 0; j < 40; j++)
+            for (int k = 0; k < 4; k++) {
+                tv[GnnW::SCALAR + L::W1tx + 8 * (j >> 1) + 2 * k + (j & 1)] = W1x[k * 40 + j];
+                tv[GnnW::SCALAR + L::W1tz + 8 * (j >> 1) + 2 * k + (j & 1)] = W1z[k * 40 + j];
+            }
         CK(cudaMalloc(&g->w_tc, tv.size() * sizeof(float)));
         CK(cudaMemcpy(g->w_tc, tv.data(), tv.size() * sizeof(float), cudaMemcpyHostToDevice));
     }

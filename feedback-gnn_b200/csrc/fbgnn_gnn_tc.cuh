@@ -31,24 +31,43 @@ struct GnnW {                                  // offsets in floats; each operan
 };
 
 // One side's edge phase of a tile row: hidden sums over the DV edges, 8 hidden units at a time, straight into TMEM as
-// the A operand of the W2 product (hi at [0, 40), lo at [40, 80)).
+// the A operand of the W2 product (hi at [0, 40), lo at [40, 80)).  The first-layer rows of units j, j+1 (j even) sit
+// interleaved in this blob, {w_cn, w_Lx, w_Ly, w_Lz} of j in the even and of j+1 in the odd positions (fbgnn_gnn.cu), so
+// that in paired arithmetic (MATH::kPaired) the two units go through the same float2 instructions with no moves.
 template <int DV, typename MATH>
-__device__ __forceinline__ void gnn_edges_tc(const Grp &g, const float *__restrict__ w1t, const float *__restrict__ b1,
+__device__ __forceinline__ void gnn_edges_tc(const Grp &g, const float *__restrict__ w1p, const float *__restrict__ b1,
                                              const float hc[DV], float f1, float f2, float f3) {
     constexpr int H = 40, JB = 8;
 #pragma unroll 1
     for (int j0 = 0; j0 < H; j0 += JB) {
         uint32_t hi[JB], lo[JB];
 #pragma unroll
-        for (int q = 0; q < JB; q++) {
-            const float4 w = *reinterpret_cast<const float4 *>(w1t + 4 * (j0 + q));      // {w_cn, w_Lx, w_Ly, w_Lz}
-            const float base = FB_FMA(f3, w.w, FB_FMA(f2, w.z, FB_FMA(f1, w.y, b1[j0 + q])));     // bias first
-            float hs = MATH::tanh(FB_FMA(hc[0], w.x, base));
+        for (int q = 0; q < JB; q += 2) {
+            const float4 wa = *reinterpret_cast<const float4 *>(w1p + 4 * (j0 + q));       // {cn_j, cn_j+1, Lx_j, Lx_j+1}
+            const float4 wb = *reinterpret_cast<const float4 *>(w1p + 4 * (j0 + q) + 4);   // {Ly_j, Ly_j+1, Lz_j, Lz_j+1}
+            float2 hs;
+            if constexpr (MATH::kPaired) {
+                const float2 wcn = make_float2(wa.x, wa.y);
+                const float2 base = FB_FMA2(fb2s(f3), make_float2(wb.z, wb.w), FB_FMA2(fb2s(f2), make_float2(wb.x, wb.y),
+                                            FB_FMA2(fb2s(f1), make_float2(wa.z, wa.w), make_float2(b1[j0 + q], b1[j0 + q + 1]))));
+                hs = MATH::tanh2(FB_FMA2(fb2s(hc[0]), wcn, base));
 #pragma unroll
-            for (int k = 1; k < DV; k++) hs = FB_ADD(hs, MATH::tanh(FB_FMA(hc[k], w.x, base)));
-            const float h = tf32_hi(hs);
-            hi[q] = __float_as_uint(h);
-            lo[q] = __float_as_uint(hs - h);
+                for (int k = 1; k < DV; k++) hs = FB_ADD2(hs, MATH::tanh2(FB_FMA2(fb2s(hc[k]), wcn, base)));
+            } else {
+                const float base0 = FB_FMA(f3, wb.z, FB_FMA(f2, wb.x, FB_FMA(f1, wa.z, b1[j0 + q])));     // bias first
+                const float base1 = FB_FMA(f3, wb.w, FB_FMA(f2, wb.y, FB_FMA(f1, wa.w, b1[j0 + q + 1])));
+                hs.x = MATH::tanh(FB_FMA(hc[0], wa.x, base0));
+                hs.y = MATH::tanh(FB_FMA(hc[0], wa.y, base1));
+#pragma unroll
+                for (int k = 1; k < DV; k++) {
+                    hs.x = FB_ADD(hs.x, MATH::tanh(FB_FMA(hc[k], wa.x, base0)));
+                    hs.y = FB_ADD(hs.y, MATH::tanh(FB_FMA(hc[k], wa.y, base1)));
+                }
+            }
+            const float2 h = make_float2(tf32_hi(hs.x), tf32_hi(hs.y));
+            const float2 l = MATH::kPaired ? FB_SUB2(hs, h) : make_float2(FB_SUB(hs.x, h.x), FB_SUB(hs.y, h.y));
+            hi[q] = __float_as_uint(h.x); hi[q + 1] = __float_as_uint(h.y);
+            lo[q] = __float_as_uint(l.x); lo[q + 1] = __float_as_uint(l.y);
         }
         __syncwarp();
         tmem_st8(g.lane_base + j0, hi);
@@ -136,6 +155,24 @@ __global__ void __launch_bounds__(256, 2) k_gnn_tc(const GnnArgs a, const float 
         for (int c0 = 0; c0 < H; c0 += 8) {
             float d[8];
             tmem_ld8(g.lane_base + 80 + c0, d);
+            if constexpr (MATH::kPaired) {          // units j, j+1 as one float2; o0 / o1 / o2 keep their j order
+#pragma unroll
+                for (int q = 0; q < 8; q += 2) {
+                    const int j = c0 + q;
+                    auto row = [&](int off) { return make_float2(ws[off + j], ws[off + j + 1]); };
+                    float2 h = FB_FMA2(fb2s(f1), row(Lay::W3 + (2 * M) * H), make_float2(d[q], d[q + 1]));
+                    h = FB_FMA2(fb2s(f2), row(Lay::W3 + (2 * M + 1) * H), h);
+                    h = FB_FMA2(fb2s(f3), row(Lay::W3 + (2 * M + 2) * H), h);
+                    h = MATH::tanh2(FB_ADD2(h, row(Lay::b3)));
+                    o0 = FB_FMA(h.x, ws[Lay::W0 + j * 3 + 0], o0);
+                    o1 = FB_FMA(h.x, ws[Lay::W0 + j * 3 + 1], o1);
+                    o2 = FB_FMA(h.x, ws[Lay::W0 + j * 3 + 2], o2);
+                    o0 = FB_FMA(h.y, ws[Lay::W0 + j * 3 + 3], o0);
+                    o1 = FB_FMA(h.y, ws[Lay::W0 + j * 3 + 4], o1);
+                    o2 = FB_FMA(h.y, ws[Lay::W0 + j * 3 + 5], o2);
+                }
+                continue;
+            }
 #pragma unroll
             for (int q = 0; q < 8; q++) {
                 const int j = c0 + q;

@@ -67,6 +67,7 @@ __device__ __forceinline__ float u01(uint32_t r) { return (float)(r >> 8) * 5.96
 struct MathExact {
     static constexpr bool kSaturationShortcuts = true;
     static constexpr bool kSharedVnCorr = false;       // the reference's per-edge logaddexp
+    static constexpr bool kPaired = false;             // FP32-pipe-bound: packed FP32 loses here (see WSmem)
     static __device__ __forceinline__ float softplus(float x) { return fb_softplusf(x); }
     static __device__ __forceinline__ float logaddexp(float a, float b) { return fb_logaddexpf(a, b); }
     static __device__ __forceinline__ float phi4(float x) { return fb_phi4f(x); }
@@ -101,6 +102,12 @@ struct MathSfu {
     static __device__ __forceinline__ float phi4_open(float x) { return fb_sfu_phi4_open(x); }
     static __device__ __forceinline__ float phi2_open(float x) { return fb_sfu_phi2_open(x); }
     static __device__ __forceinline__ float logaddexp_open(float mx, float d) { return fb_sfu_logaddexp_open(mx, d); }
+    // issue-bound: the independent FP32 operations of the hot loops go two per instruction (fb_math.h paired forms)
+    static constexpr bool kPaired = true;
+    static __device__ __forceinline__ float2 phi_open2(float2 x) { return fb_sfu_phi_open2(x); }
+    static __device__ __forceinline__ float2 softplus2(float2 x) { return fb_sfu_softplusf2(x); }
+    static __device__ __forceinline__ float2 logaddexp_open2(float2 mx, float2 d) { return fb_sfu_logaddexp_open2(mx, d); }
+    static __device__ __forceinline__ float2 tanh2(float2 x) { return fb_sfu_tanhf2(x); }
 };
 
 // Lab knobs (make lab ..., tools/lab_bench.py): compile-time experiments, all bit-exact.  Measured on B200
@@ -181,8 +188,17 @@ __device__ __forceinline__ void phi_sat_group(const float x[G], float r[G]) {
         need = need || !sat[k];
     }
     if (!FBGNN_VOTE || __any_sync(FULL ? 0xffffffffu : __activemask(), need)) {
+        int k0 = 0;
+        if constexpr (MATH::kPaired && FBGNN_LEAN) {         // sites 2i, 2i+1 as one float2 evaluation (odd G: the last alone)
 #pragma unroll
-        for (int k = 0; k < G; k++) {
+            for (; k0 + 1 < G; k0 += 2) {
+                const float2 f = MATH::phi_open2(make_float2(x[k0], x[k0 + 1]));
+                r[k0] = sat[k0] ? r[k0] : f.x;
+                r[k0 + 1] = sat[k0 + 1] ? r[k0 + 1] : f.y;
+            }
+        }
+#pragma unroll
+        for (int k = k0; k < G; k++) {
             const float f = phi_eval<MATH, PHI4>(x[k]);
             r[k] = sat[k] ? r[k] : f;
         }
@@ -229,15 +245,28 @@ __device__ __forceinline__ void logaddexp_sat_group(const float a[G], const floa
 }
 
 // SFU arithmetic: the two edge-independent terms of a variable node's outgoing messages (fb_math.h fb_sfu_vn_corr), the x
-// edges' (from lz, ly) and the z edges' (from lx, ly), evaluated under one warp vote.
-template <typename MATH, bool FULL>
+// edges' (from lz, ly) and the z edges' (from lx, ly), evaluated under one warp vote.  PAIRED: the two as one float2
+// evaluation (the regular fast path in paired arithmetic).
+template <typename MATH, bool FULL, bool PAIRED = false>
 __device__ __forceinline__ void vn_corr_pair(float lx, float ly, float lz, float &ux, float &cx, float &uz, float &cz) {
     ux = fminf(lz, ly); uz = fminf(lx, ly);
-    const float dx = -fabsf(FB_SUB(ly, lz)), dz = -fabsf(FB_SUB(ly, lx));
+    float dx, dz;
+    if constexpr (PAIRED) {
+        const float2 d = FB_SUB2(make_float2(ly, ly), make_float2(lz, lx));
+        dx = -fabsf(d.x); dz = -fabsf(d.y);
+    } else {
+        dx = -fabsf(FB_SUB(ly, lz)); dz = -fabsf(FB_SUB(ly, lx));
+    }
     const bool satx = dx < -17.5f, satz = dz < -17.5f;
     cx = 0.0f; cz = 0.0f;
     if (!FBGNN_VOTE || __any_sync(FULL ? 0xffffffffu : __activemask(), !(satx && satz))) {
-        const float fx = MATH::logaddexp_open(0.0f, dx), fz = MATH::logaddexp_open(0.0f, dz);
+        float fx, fz;
+        if constexpr (PAIRED) {
+            const float2 f = MATH::logaddexp_open2(make_float2(0.0f, 0.0f), make_float2(dx, dz));
+            fx = f.x; fz = f.y;
+        } else {
+            fx = MATH::logaddexp_open(0.0f, dx); fz = MATH::logaddexp_open(0.0f, dz);
+        }
         cx = satx ? 0.0f : fx; cz = satz ? 0.0f : fz;
     }
 }
@@ -380,18 +409,30 @@ __device__ __forceinline__ bool cn_phi_regular(const idx_t *__restrict__ cn_edge
     for (int k = 0; k < DC; k++) T = FB_ADD(T, a[k]);
     bool stable = FPX && rec != nullptr;
     float xo[DC], vo[DC];
+    constexpr int NP = MATH::kPaired ? DC / 2 : 0;  // sites 2i, 2i+1 paired (odd DC: the last alone)
 #pragma unroll
-    for (int k = 0; k < DC; k++) xo[k] = FB_SUB(T, a[k]);
+    for (int i = 0; i < NP; i++) {
+        const float2 x2 = FB_SUB2(make_float2(T, T), make_float2(a[2 * i], a[2 * i + 1]));
+        xo[2 * i] = x2.x; xo[2 * i + 1] = x2.y;
+    }
+#pragma unroll
+    for (int k = 2 * NP; k < DC; k++) xo[k] = FB_SUB(T, a[k]);
 #pragma unroll
     for (int k = 0; k < DC; k += GRP) phi_sat_group<MATH, PHI4, GRP, FULL>(xo + k, vo + k);
     bool allsat = true;
     uint32_t sw[DC];                                // sign of the outgoing message, in the sign position
+    float v[DC];
 #pragma unroll
     for (int k = 0; k < DC; k++) {
         sw[k] = SIGNBITS ? ((word[k] & 0x80000000u) ^ pw) : ((((uint32_t)par ^ (neg >> k)) & 1u) << 31);
-        const float v = __int_as_float(__float_as_int(vo[k]) ^ (int)sw[k]);
-        msg[e[k]] = FB_MUL(v, factor);
+        v[k] = __int_as_float(__float_as_int(vo[k]) ^ (int)sw[k]);
         allsat = allsat && (xo[k] <= FB_PHI_CLIP_LO);
+        if (k < 2 * NP && (k & 1)) {
+            const float2 m2 = FB_MUL2(make_float2(v[k - 1], v[k]), make_float2(factor, factor));
+            msg[e[k - 1]] = m2.x; msg[e[k]] = m2.y;
+        } else if (k >= 2 * NP) {
+            msg[e[k]] = FB_MUL(v[k], factor);
+        }
     }
     if (FPX && rec) {
         // one vote per check: only the AND over the whole frame is used (k_bp4's __syncthreads_and), so a warp with
@@ -429,6 +470,24 @@ __device__ __forceinline__ void vn_update_regular(int v, float *mx, float *mz, f
             bad |= ((bx & 0x7fffffff) ^ sat_bits) | ((bz & 0x7fffffff) ^ sat_bits);
         }
         rec[v] = (uint16_t)(bad ? 0x8000 : r);
+    }
+    if constexpr (MATH::kPaired && MATH::kSharedVnCorr) {
+        // lane x: the x edges' chain, lane y: the z edges' -- the two sums keep their order, each message is vn_msg
+        float2 S = make_float2(0.0f, 0.0f);
+#pragma unroll
+        for (int k = 0; k < DV; k++) S = FB_ADD2(S, make_float2(ax[k], az[k]));
+        const float ly = FB_ADD(FB_ADD(S.y, S.x), py);
+        const float2 l = FB_ADD2(make_float2(S.y, S.x), make_float2(px, pz));         // (lx, lz)
+        const float2 num = MATH::softplus2(fb2_neg(l));
+        float ux, cx, uz, cz;
+        vn_corr_pair<MATH, FULL, true>(l.x, ly, l.y, ux, cx, uz, cz);
+#pragma unroll
+        for (int k = 0; k < DV; k++) {
+            const float2 m = fb_sfu_vn_msg2(num, make_float2(ax[k], az[k]), make_float2(ux, uz), make_float2(cx, cz));
+            mx[v * DV + k] = m.x;
+            mz[v * DV + k] = m.y;
+        }
+        return;
     }
     float Sx = 0.0f, Sz = 0.0f;
 #pragma unroll
@@ -616,8 +675,12 @@ __device__ void bp4_iter_logits(const Bp4Args &a, const float *mx, const float *
 //   iter_logits);  u16 rec[n];  u8 dec[n]
 // GSTATE (codes whose state exceeds the 227 KB of an SM): the float arrays live in the CTA's slice of an HBM
 // scratch buffer (L2-resident while the CTA runs) instead; same code, same arithmetic, same results.
+// Paired arithmetic on (3,6) / (4,8) codes: at least 2 CTAs of 512 threads, i.e. up to 64 registers.  Left alone, ptxas
+// aims at 3 CTAs of 512 (40 registers), where the paired regular path spills.  On [[1270,28]] the launcher runs 256
+// threads per CTA and shared memory allows 4 CTAs per SM, which 64 registers still allow (4 x 256 x 64 = 65 536).
+// (5,10) needs more than 64 registers and keeps ptxas's choice.
 template <bool CONST_PRIOR, int DV, int DC, typename MATH, bool FPX, bool GSTATE = false>
-static __global__ void __launch_bounds__(512) k_bp4(const Bp4Args a) {
+static __global__ void __launch_bounds__(512, (MATH::kPaired && DV > 0 && DV <= 4) ? 2 : 0) k_bp4(const Bp4Args a) {
     extern __shared__ __align__(16) float smem[];
     __shared__ __align__(8) uint64_t load_bar;
     const SideDev &X = a.X, &Z = a.Z;
@@ -1032,7 +1095,10 @@ __device__ __forceinline__ float gnn_act(int act, float x) {
 
 // Weights staged per CTA in shared memory and read as broadcast loads.  (Measured alternative:
 // __constant__ memory through LDC is 19 % slower for this kernel -- higher load latency, same FFMA
-// operand traffic -- and packed fma.rn.f32x2 sustains only 0.77x the lanes/s of scalar FFMA on B200.)
+// operand traffic.)  Packed fma.rn.f32x2 sustains only 0.77x the lanes/s of scalar FFMA on B200
+// (tools/micro/ffma2_bench.cu), so it loses wherever the FP32 pipe is the limit -- this kernel, and
+// the exact arithmetic (MathExact::kPaired = false).  It wins where instruction issue is the limit
+// and the FP32 pipe has room: the SFU kernels (MathSfu::kPaired).
 struct WSmem {
     const float *p;
     __device__ __forceinline__ float ld(int i) const { return p[i]; }
@@ -2459,12 +2525,44 @@ static __global__ void k_final(const FinalArgs a) {
 }
 
 // ------------------------------------------------------------------ probes ------------
+// Functions of several arguments take them from the input at the element's index and at three others (the same for the
+// scalar and the paired form).  Paired forms (fn >= 25) evaluate elements 2i and 2i+1 as the two lanes of one call.
+struct ProbeArgs {
+    float a0, a1, a2, a3;
+    __device__ ProbeArgs(const float *x, int64_t n, int64_t i)
+        : a0(x[i]), a1(x[n - 1 - i]), a2(x[(i + n / 3) % n]), a3(x[(i + 2 * (n / 3)) % n]) {}
+};
 static __global__ void k_math_probe(int fn, const float *x, float *y, int64_t n) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
+    if (fn >= 25) {
+        if (i & 1) return;
+        const int64_t i1 = i + 1 < n ? i + 1 : i;
+        const ProbeArgs p(x, n, i), q(x, n, i1);
+        const float2 a0 = make_float2(p.a0, q.a0), a1 = make_float2(p.a1, q.a1);
+        float2 r;
+        switch (fn) {
+            case 25: r = fb_sfu_exp2s2(a0, -FB_LOG2E); break;
+            case 26: r = fb_sfu_logaddexp_open2(a0, a1); break;
+            case 27: r = fb_sfu_vn_corr2(a0, a1); break;
+            case 28: r = fb_sfu_vn_msg2(a0, a1, make_float2(p.a2, q.a2), make_float2(p.a3, q.a3)); break;
+            case 29: r = fb_sfu_phi_open2(a0); break;
+            case 30: r = fb_sfu_softplusf2(a0); break;
+            default: r = fb_sfu_tanhf2(a0); break;
+        }
+        y[i] = r.x;
+        if (i1 != i) y[i1] = r.y;
+        return;
+    }
     const float v = x[i];
     float r;
+    const ProbeArgs p(x, n, i);
     switch (fn) {
+        case 20: r = fb_sfu_exp2s(v, -FB_LOG2E); break;
+        case 21: r = fb_sfu_logaddexp_open(p.a0, p.a1); break;
+        case 22: r = fb_sfu_vn_corr(p.a0, p.a1); break;
+        case 23: r = fb_sfu_vn_msg(p.a0, p.a1, p.a2, p.a3); break;
+        case 24: r = fb_sfu_phi_open(v); break;
         case 0: r = fb_expf(v); break;
         case 1: r = fb_logf(v); break;
         case 2: r = fb_log1pf_pos(v); break;
