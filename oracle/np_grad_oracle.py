@@ -1,11 +1,13 @@
 """TEST INFRASTRUCTURE -- float64 numpy restatement of the loss of Second_Stage_GNN_BP_Model.call
 (sionna/fec/ldpc/feedback_gnn.py:412-431: Feedback_GNN -> QLDPCBPDecoder(stage_two) -> multi-loss BCE), used
-to check the hand-written gradient of csrc/fbgnn_train.cuh by central finite differences.
+to check the hand-written gradient of csrc/fbgnn_train.cuh.
 
 Only tests/ may import this module.  Everything is evaluated with the exact mathematical functions in
 float64 (no float32 thresholds), so it is the smooth function whose derivative the CUDA reverse sweep
-approximates at float32 accuracy.  Parity of the gradient with the reference is UNPINNED (TensorFlow is not
-available); the pins are finite differences of this restatement.
+approximates at float32 accuracy.  Parity of the gradient with TensorFlow is unpinned (TensorFlow is not
+available).  oracle/torch_grad_oracle.py restates this loss in torch (equal to 1e-12, reduce "sum" added) and
+differentiates it by autograd; tests/test_train_grad.py compares the CUDA gradient with that, array by array and
+element by element (profiles/grad_error_b200.txt).
 """
 import numpy as np
 

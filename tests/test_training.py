@@ -2,9 +2,11 @@
 (feedback_gnn.py:364-460), the gradient tf.GradientTape would return, Adam, and the dataset generators of
 examples/Generate_dataset.ipynb.
 
-Parity of the gradient with the reference is UNPINNED (no TensorFlow in the image, no recorded gradients in the
-repository).  The pins are: the loss against the float64 numpy restatement oracle/np_grad_oracle.py, and the
-gradient against central finite differences of that restatement."""
+Parity of the gradient with TensorFlow is unpinned (no TensorFlow in the image, no recorded gradients in the
+repository).  Here: the loss against the float64 numpy restatement oracle/np_grad_oracle.py, and the gradient
+against central finite differences of that restatement.  The element-by-element pin of the gradient against a float64
+autograd reference (oracle/torch_grad_oracle.py) over many codes, batch sizes and configurations is
+tests/test_train_grad.py."""
 import numpy as np
 import pytest
 
