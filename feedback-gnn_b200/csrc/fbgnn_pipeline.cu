@@ -1,6 +1,7 @@
 // fbgnn_pipeline.cu -- the fused Monte-Carlo pipelines (multi-launch orchestration) and OSD.
 #include "fbgnn_internal.h"
 #include "fbgnn_osd_cluster.cuh"
+#include "fbgnn_lsd.cuh"
 
 // ------------------------------------------------------------------ OSD -----------------
 // Dynamic shared memory of one OSD CTA that holds `rows` basis rows; with `cluster`, the layout of k_osd_cluster (its
@@ -111,6 +112,44 @@ extern "C" int fbgnn_osd0_decode(fbgnn_graph *basis, int64_t B, fbgnn_tensor2 ll
     return fbgnn_osd_decode(basis, 0, B, llr, synd, e_hat);
 }
 
+// ------------------------------------------------------------------ LSD-0 ---------------
+// Budgets: 0 = the default; otherwise [1, limit].  The limits keep the worst case (n = m = 65535) inside one CTA.
+static int lsd_budgets(int32_t *max_cols, int32_t *max_checks) {
+    if (*max_cols == 0) *max_cols = LSD_DEF_COLS;
+    if (*max_checks == 0) *max_checks = LSD_DEF_CHECKS;
+    REQUIRE(*max_cols >= 1 && *max_cols <= LSD_MAX_COLS, "LSD max_cols %d outside [1, %d]", *max_cols, LSD_MAX_COLS);
+    REQUIRE(*max_checks >= 1 && *max_checks <= LSD_MAX_CHECKS, "LSD max_checks %d outside [1, %d]", *max_checks,
+            LSD_MAX_CHECKS);
+    return 0;
+}
+
+static int launch_lsd(fbgnn_ctx *ctx, LsdArgs &a, int64_t grid) {
+    if (grid <= 0) return 0;
+    const size_t smem = LsdLayout(a.S.n, a.S.m, a.max_cols, a.max_checks).total;
+    if (int rc = set_smem(k_lsd, smem, ctx, "LSD-0")) return rc;
+    k_lsd<<<(unsigned)grid, 256, smem, ctx->stream>>>(a);
+    CK(cudaGetLastError());
+    ctx->launches++;
+    return 0;
+}
+
+extern "C" int fbgnn_lsd_decode(fbgnn_graph *pcm, int32_t max_cols, int32_t max_checks, int64_t B, fbgnn_tensor2 llr,
+                                fbgnn_tensor2 synd, fbgnn_tensor2 e_hat, uint8_t *status) {
+    REQUIRE(pcm && llr.ptr && synd.ptr && B >= 0 && B < ((int64_t)1 << 31), "bad argument");
+    if (int rc = lsd_budgets(&max_cols, &max_checks)) return rc;
+    if (int rc = need_decodable(pcm)) return rc;
+    fbgnn_ctx *ctx = pcm->ctx;
+    if (set_device(ctx)) return FBGNN_E_CUDA;
+    LsdArgs a{};
+    a.S = pcm->dev;
+    a.llr = v2<const float>(llr); a.sign = 1.0f;
+    a.synd = v2<const uint8_t>(synd);
+    a.e_hat = v2<uint8_t>(e_hat);
+    a.status = status;
+    a.max_cols = max_cols; a.max_checks = max_checks;
+    return launch_lsd(ctx, a, B);
+}
+
 // ------------------------------------------------------------------ pipelines -----------
 static int ws_reserve(fbgnn_ctx *ctx, int64_t B, int n, int m) {
     Workspace &w = ctx->ws;
@@ -172,8 +211,11 @@ static int pipeline_run_impl(fbgnn_code *code, const fbgnn_pipeline_cfg *cfg, ui
     REQUIRE(cfg->num_stages == 1 || cfg->gnn, "feedback GNNs missing");
     REQUIRE((noise_x.ptr == nullptr) == (noise_z.ptr == nullptr), "give both noise_x and noise_z or neither");
     REQUIRE(B >= 0 && B < ((int64_t)1 << 31), "bad batch size");
-    REQUIRE(!cfg->osd0 || (code->basis_x && code->basis_z), "OSD-0 needs fbgnn_code_set_basis first");
+    REQUIRE(!cfg->osd0 || cfg->lsd || (code->basis_x && code->basis_z), "OSD-0 needs fbgnn_code_set_basis first");
     if (int rc = check_osd_order(cfg->osd_order)) return rc;
+    int32_t lsd_cols = cfg->lsd_max_cols, lsd_checks = cfg->lsd_max_checks;
+    if (cfg->osd0 && cfg->lsd)
+        if (int rc = lsd_budgets(&lsd_cols, &lsd_checks)) return rc;
     REQUIRE(cfg->fixed_weight <= 0 || code->X->dev.n <= 65535, "fixed-weight sampling shuffles uint16 qubit indices (n <= 65535)");
     for (int s = 0; s < cfg->num_stages; s++) {
         REQUIRE(cfg->cn_type[s] >= 0 && cfg->cn_type[s] <= 2, "unknown cn_type in stage %d", s);
@@ -274,6 +316,21 @@ static int pipeline_run_impl(fbgnn_code *code, const fbgnn_pipeline_cfg *cfg, ui
         else k_osd_llr<MathExact><<<(unsigned)blocks, 256, 0, st>>>(la);
         CK(cudaGetLastError());
         ctx->launches++;
+        if (cfg->lsd) {
+            // LSD-0 on each side's full matrix; a side it abandons keeps its BP decision
+            LsdArgs ls{};
+            ls.frame_list = cur_list; ls.sign = 1.0f;
+            ls.vbits = w.vbits;
+            ls.max_cols = lsd_cols; ls.max_checks = lsd_checks;
+            ls.S = X;                                                    // hx, osd_llrz, syndrome_x -> z_hat
+            ls.llr = View2<const float>{w.P + np, 3 * (int64_t)np, 1};
+            ls.synd = View2<const uint8_t>{w.sbits, 1, mp}; ls.vbit = 3;
+            if (int rc = launch_lsd(ctx, ls, cur_count)) return rc;
+            ls.S = Z;                                                    // hz, osd_llrx, syndrome_z -> x_hat
+            ls.llr = View2<const float>{w.P, 3 * (int64_t)np, 1};
+            ls.synd = View2<const uint8_t>{w.sbits + X.m, 1, mp}; ls.vbit = 2;
+            if (int rc = launch_lsd(ctx, ls, cur_count)) return rc;
+        } else {
         OsdArgs oa{};
         oa.frame_list = cur_list; oa.sign = 1.0f;
         oa.vbits = w.vbits;
@@ -285,6 +342,7 @@ static int pipeline_run_impl(fbgnn_code *code, const fbgnn_pipeline_cfg *cfg, ui
         oa.llr = View2<const float>{w.P, 3 * (int64_t)np, 1};
         oa.synd = View2<const uint8_t>{w.sbits + X.m, 1, mp}; oa.synd_row = code->pivot_z; oa.vbit = 2;
         if (int rc = launch_osd(ctx, oa, cfg->osd_order, cur_count)) return rc;
+        }
     }
 
     FinalArgs fa{};
@@ -320,11 +378,15 @@ extern "C" int fbgnn_bsc_pipeline_run(fbgnn_graph *g, fbgnn_graph *logical, int3
                                      flags, counters, osd_basis, osd_pivot, 0);
 }
 
-extern "C" int fbgnn_bsc_pipeline_run_ex(fbgnn_graph *g, fbgnn_graph *logical, int32_t cn_type, int32_t num_iter,
-                                         float factor, float llr_const, float p, uint64_t seed, uint64_t first_frame,
-                                         int64_t B, fbgnn_tensor2 noise, uint8_t *flags, int64_t *counters,
-                                         fbgnn_graph *osd_basis, const int32_t *osd_pivot, int32_t osd_order) {
+// BP_BSC_Model with, on the frames BP2 leaves mismatching, OSD on osd_basis or (lsd) LSD-0 on g itself
+static int bsc_pipeline_impl(fbgnn_graph *g, fbgnn_graph *logical, int32_t cn_type, int32_t num_iter, float factor,
+                             float llr_const, float p, uint64_t seed, uint64_t first_frame, int64_t B,
+                             fbgnn_tensor2 noise, uint8_t *flags, int64_t *counters, fbgnn_graph *osd_basis,
+                             const int32_t *osd_pivot, int32_t osd_order, bool lsd, int32_t lsd_cols,
+                             int32_t lsd_checks) {
     REQUIRE(g, "graph is NULL");
+    if (lsd)
+        if (int rc = lsd_budgets(&lsd_cols, &lsd_checks)) return rc;
     if (int rc = check_osd_order(osd_order)) return rc;
     REQUIRE(!osd_basis || (osd_pivot && osd_basis->dev.n == g->dev.n && osd_basis->dev.m <= g->dev.m),
             "bad OSD-0 basis");
@@ -357,13 +419,24 @@ extern "C" int fbgnn_bsc_pipeline_run_ex(fbgnn_graph *g, fbgnn_graph *logical, i
     a.llr_const = llr_const;
     a.synd = View2<const uint8_t>{w.sbits, 1, mp};
     a.vbits = w.vbits;                 // decision -> bit 2
-    if (osd_basis) {
+    if (osd_basis || lsd) {
         CK(cudaMemsetAsync(w.list_count, 0, sizeof(int), st));
         a.soft = View2<float>{w.L, n, 1};
         a.next_list = w.list[0]; a.next_count = w.list_count;
     }
     if (int rc = launch_bp2(ctx, a, B)) return rc;
-    if (osd_basis) {
+    if (lsd) {
+        int cnt = 0;
+        CK(cudaMemcpyAsync(&cnt, w.list_count, sizeof(int), cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        LsdArgs ls{};
+        ls.S = S; ls.frame_list = w.list[0];
+        ls.llr = View2<const float>{w.L, n, 1}; ls.sign = -1.0f;         // llr_hat = -decoder output
+        ls.synd = View2<const uint8_t>{w.sbits, 1, mp};
+        ls.vbits = w.vbits; ls.vbit = 2;
+        ls.max_cols = lsd_cols; ls.max_checks = lsd_checks;
+        if (int rc = launch_lsd(ctx, ls, cnt)) return rc;
+    } else if (osd_basis) {
         // BP2_OSD_Model (bp_osd.py:199-274): OSD-0 on the frames whose decision misses the syndrome
         if (int rc = need_decodable(osd_basis)) return rc;
         int cnt = 0;
@@ -408,3 +481,18 @@ extern "C" int fbgnn_bsc_pipeline_run_ex(fbgnn_graph *g, fbgnn_graph *logical, i
     return 0;
 }
 
+extern "C" int fbgnn_bsc_pipeline_run_ex(fbgnn_graph *g, fbgnn_graph *logical, int32_t cn_type, int32_t num_iter,
+                                         float factor, float llr_const, float p, uint64_t seed, uint64_t first_frame,
+                                         int64_t B, fbgnn_tensor2 noise, uint8_t *flags, int64_t *counters,
+                                         fbgnn_graph *osd_basis, const int32_t *osd_pivot, int32_t osd_order) {
+    return bsc_pipeline_impl(g, logical, cn_type, num_iter, factor, llr_const, p, seed, first_frame, B, noise, flags,
+                             counters, osd_basis, osd_pivot, osd_order, false, 0, 0);
+}
+
+extern "C" int fbgnn_bsc_pipeline_run_lsd(fbgnn_graph *g, fbgnn_graph *logical, int32_t cn_type, int32_t num_iter,
+                                          float factor, float llr_const, float p, uint64_t seed, uint64_t first_frame,
+                                          int64_t B, fbgnn_tensor2 noise, uint8_t *flags, int64_t *counters,
+                                          int32_t max_cols, int32_t max_checks) {
+    return bsc_pipeline_impl(g, logical, cn_type, num_iter, factor, llr_const, p, seed, first_frame, B, noise, flags,
+                             counters, nullptr, nullptr, 0, true, max_cols, max_checks);
+}

@@ -35,7 +35,8 @@ class PipelineCfg(C.Structure):
                 ("factor", C.POINTER(C.c_float)), ("cn_type", C.POINTER(C.c_int32)),
                 ("gnn", C.POINTER(C.c_void_p)), ("prior", C.c_float), ("thr", C.c_float * 3),
                 ("fixed_weight", C.c_int32), ("osd0", C.c_int32), ("skip_inactive", C.c_int32),
-                ("early_stop", C.c_int32), ("osd_order", C.c_int32)]
+                ("early_stop", C.c_int32), ("osd_order", C.c_int32), ("lsd", C.c_int32),
+                ("lsd_max_cols", C.c_int32), ("lsd_max_checks", C.c_int32)]
 
 
 class Bp4Opts(C.Structure):
@@ -96,6 +97,7 @@ _SIGNATURES = {
                             Tensor2, C.c_void_p, Tensor2, Tensor2],
     "fbgnn_osd0_decode": [C.c_void_p, C.c_int64, Tensor2, Tensor2, Tensor2],
     "fbgnn_osd_decode": [C.c_void_p, C.c_int32, C.c_int64, Tensor2, Tensor2, Tensor2],
+    "fbgnn_lsd_decode": [C.c_void_p, C.c_int32, C.c_int32, C.c_int64, Tensor2, Tensor2, Tensor2, C.c_void_p],
     "fbgnn_gnn_create": [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32] + [_f32p] * 12 + [_vpp],
     "fbgnn_gnn_create_deep": [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _f32p,
                               C.c_int64, _vpp],
@@ -122,6 +124,9 @@ _SIGNATURES = {
     "fbgnn_bsc_pipeline_run_ex": [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_float, C.c_float, C.c_float,
                                   C.c_uint64, C.c_uint64, C.c_int64, Tensor2, C.c_void_p, C.POINTER(C.c_int64),
                                   C.c_void_p, _i32p, C.c_int32],
+    "fbgnn_bsc_pipeline_run_lsd": [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_float, C.c_float, C.c_float,
+                                   C.c_uint64, C.c_uint64, C.c_int64, Tensor2, C.c_void_p, C.POINTER(C.c_int64),
+                                   C.c_int32, C.c_int32],
     "fbgnn_comm_unique_id": [C.POINTER(C.c_uint8)],
     "fbgnn_comm_init_rank": [C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_uint8)],
     "fbgnn_comm_info": [C.c_void_p, _i32p, _i32p, _i32p],

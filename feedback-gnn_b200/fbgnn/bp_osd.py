@@ -1,4 +1,4 @@
-"""BP + OSD post-processing -- ``OSD_Decoder``, ``OSD0_Decoder``, ``BP4_OSD_Model``, ``BP2_OSD_Model``.
+"""BP + OSD post-processing -- ``OSD_Decoder``, ``OSD0_Decoder``, ``LSD_Decoder``, ``BP4_OSD_Model``, ``BP2_OSD_Model``.
 
 Mirrors ``sionna/fec/ldpc/bp_osd.py`` of the reference: the frames whose BP decision misses the
 syndrome are re-solved by ordered-statistics decoding of order 0 (``:8-77``): columns ordered by the
@@ -20,6 +20,12 @@ A frame's reduced matrix sits in the shared memory of one CTA (``k_osd``).  Wher
 [[1922,50]] hypergraph-product code, a thread-block cluster of 2, 4 or 8 CTAs splits it by rows (``k_osd_cluster``,
 the same result bit for bit).  A basis beyond a cluster of 8 (about 1.8 MB, e.g. [[7688,50]]) raises ``FbgnnError``
 with ``FBGNN_E_UNSUPPORTED`` (-3).
+
+``LSD_Decoder(n, max_cols, max_checks)`` is localised statistics decoding of order 0 (LSD-0; Hillmann et al. 2024, the
+``ldpc`` package's ``BpLsdDecoder``, ``k_lsd``): instead of eliminating the whole matrix it grows clusters around the
+unsatisfied checks, least reliable column first, until each cluster explains its own syndrome, and solves each cluster
+as OSD-0 would.  Its cost depends on the cluster sizes, not on n, so it runs on every code, [[7688,50]] included; a
+frame whose clusters outgrow the budgets is abandoned (``last_status`` 1, e_hat = 0).
 """
 import numpy as np
 
@@ -81,6 +87,45 @@ class OSD0_Decoder(OSD_Decoder):
         super().__init__(n, osd_order=0, osd_method="osd0", ctx=ctx)
 
 
+class LSD_Decoder:
+    """``LSD_Decoder(n, max_cols=0, max_checks=0)(llr [bs,n], pcm [m,n] (or [bs,m,n]), s [m,bs], bs) -> e_hat [bs,n]``
+    bool: LSD-0 on the parity-check matrix ``pcm`` itself (the full hx / hz, or an OSD basis with the reduced syndrome).
+    The budgets bound the columns / checks of all clusters of a frame together: 0 = the defaults (256 / 256), at most
+    512 each.  ``last_status`` holds the status of every frame of the last call (uint8 [bs]): 0 solved, 1 abandoned
+    over budget, 2 abandoned because s is outside the column space of ``pcm``; abandoned frames get e_hat = 0."""
+
+    MAX_COLS = MAX_CHECKS = 512
+
+    def __init__(self, n, max_cols=0, max_checks=0, ctx=None):
+        max_cols, max_checks = int(max_cols), int(max_checks)
+        if not 0 <= max_cols <= self.MAX_COLS or not 0 <= max_checks <= self.MAX_CHECKS:
+            raise ValueError(f"max_cols / max_checks must be in [0, 512] (0 = default), got {max_cols} / {max_checks}")
+        self.n, self.max_cols, self.max_checks = int(n), max_cols, max_checks
+        self._ctx = ctx
+        self._graphs = {}
+        self.last_status = None
+
+    _graph = OSD_Decoder._basis_graph
+
+    def __call__(self, llr, pcm, s, bs=None):
+        g = self._graph(pcm)
+        ctx = g.ctx
+        on_device = _is_device(llr) or _is_device(s)
+        llr_d = ctx.asarray(llr, np.float32)
+        B = llr_d.shape[0]
+        s_d = ctx.asarray(_to_u8(s), np.uint8)
+        if llr_d.shape != (B, self.n) or g.n != self.n or s_d.shape != (g.m, B):
+            raise ValueError(f"expected llr [bs,{self.n}], pcm [m,{self.n}], s [m,bs]")
+        e_hat = ctx.empty((B, self.n), np.uint8)
+        status = ctx.empty((B,), np.uint8)
+        _ffi.call("fbgnn_lsd_decode", g.handle, self.max_cols, self.max_checks, B, llr_d.t2(), s_d.t2(), e_hat.t2(),
+                  status.ptr)
+        self.last_status = status if on_device else status.numpy()
+        return e_hat if on_device else e_hat.numpy().astype(bool)
+
+    call = __call__
+
+
 def _osd_order(osd_decoder):
     return int(getattr(osd_decoder, "osd_order", 0))
 
@@ -103,16 +148,19 @@ def _indicators(flags, rows, dense=None):
 
 class BP4_OSD_Model:
     """Quaternary BP followed by OSD on the failed frames (bp_osd.py:80-197), of the order of ``osd_decoder``
-    (``OSD0_Decoder``: OSD-0).  The prior is log(3(1-p)/p) with the simulated p (``:121``)."""
+    (``OSD0_Decoder``: OSD-0), or by LSD-0 on each side's full matrix when ``osd_decoder`` is an ``LSD_Decoder``.  The
+    prior is log(3(1-p)/p) with the simulated p (``:121``)."""
 
     def __init__(self, code, bp4_decoder, osd_decoder, seed=0, first_frame=0, ctx=None):
         if not isinstance(bp4_decoder, QLDPCBPDecoder):
             raise TypeError("bp4_decoder must be an fbgnn QLDPCBPDecoder layer")
         self.code, self.k, self.n = code, code.K, code.N
         self.bp4_decoder, self.osd_decoder = bp4_decoder, osd_decoder
+        lsd = osd_decoder if isinstance(osd_decoder, LSD_Decoder) else None
         self._inner = Sandwich_BP_GNN_Evaluation_Model(code, [bp4_decoder], [], num_layers=1, p0=None, seed=seed,
-                                                       first_frame=first_frame, osd0=True,
-                                                       osd_order=_osd_order(osd_decoder), ctx=ctx)
+                                                       first_frame=first_frame, osd0=lsd is None,
+                                                       osd_order=0 if lsd else _osd_order(osd_decoder), ctx=ctx,
+                                                       lsd=lsd)
 
     @property
     def last_counters(self):
@@ -136,7 +184,8 @@ class BP4_OSD_Model:
 
 class BP2_OSD_Model:
     """Binary syndrome BP on a BSC followed by OSD on the failed frames (bp_osd.py:199-274), of the order of
-    ``osd_decoder``; the BP logit is -log((1-p)/p) with the simulated p (``:221``)."""
+    ``osd_decoder``; the BP logit is -log((1-p)/p) with the simulated p (``:221``).  With an ``LSD_Decoder`` the failed
+    frames are re-solved by LSD-0 on ``pcm`` itself, and ``pcm_basis`` / ``pivot_pcm`` are unused."""
 
     def __init__(self, pcm, pcm_basis, pivot_pcm, logical_pcm, bp2_decoder, osd_decoder, seed=0, first_frame=0,
                  ctx=None):
@@ -158,7 +207,9 @@ class BP2_OSD_Model:
 
     def run(self, batch_size, p, **kw):
         inner = self._inner
-        if inner._osd_basis is None:
+        if isinstance(self.osd_decoder, LSD_Decoder):
+            inner._lsd = self.osd_decoder
+        elif inner._osd_basis is None:
             g, _ = inner._graphs()
             inner._osd_basis = _ffi.Graph(self.pcm_basis, g.ctx)
             inner._osd_pivot = self.pivot_pcm

@@ -265,10 +265,13 @@ class Sandwich_BP_GNN_Evaluation_Model:
                       reproduces the syndrome (SURVEY.md H8).  NOT what the reference computes -- it always runs
                       num_iter iterations -- so it is off by default and excluded from parity claims
       osd_order       with osd0: 0 runs OSD-0, λ > 0 the combination sweep OSD-CS of order λ (bp_osd.OSD_Decoder)
+      lsd             a bp_osd.LSD_Decoder: the frames still mismatching after the last stage are re-solved by LSD-0 on
+                      each side's full matrix, with its budgets; a side LSD-0 abandons keeps its BP decision.  Not
+                      together with osd0=True
     """
 
     def __init__(self, code, decoders, feedbacks, num_layers=4, wt=False, p0=0.05, seed=0, first_frame=0,
-                 skip_inactive=False, osd0=False, ctx=None, early_stop=False, osd_order=0):
+                 skip_inactive=False, osd0=False, ctx=None, early_stop=False, osd_order=0, lsd=None):
         self.k, self.n = code.K, code.N
         self.code = code
         self.hx, self.hz, self.lx, self.lz = code.hx, code.hz, code.lx, code.lz
@@ -299,6 +302,13 @@ class Sandwich_BP_GNN_Evaluation_Model:
         self.osd_order = int(osd_order)
         if not 0 <= self.osd_order <= 65535:
             raise ValueError(f"osd_order must be in [0, 65535], got {osd_order}")
+        if lsd is not None:
+            from .bp_osd import LSD_Decoder
+            if not isinstance(lsd, LSD_Decoder):
+                raise TypeError("lsd must be an fbgnn LSD_Decoder")
+            if self.osd0:
+                raise ValueError("give osd0=True or lsd, not both")
+        self.lsd = lsd
         self._ctx = ctx
         self.last_counters = None
 
@@ -317,9 +327,12 @@ class Sandwich_BP_GNN_Evaluation_Model:
         gh = (C.c_void_p * max(S - 1, 1))(*[g.device_handle(ctx).value for g in self.feedbacks[:S - 1]])
         # wt=True: `p` is the error weight (feedback_gnn.py:300-301) and p0 must be given
         thr = pauli_thresholds(0.0 if self.wt else float(p))
+        lsd = self.lsd
         cfg = _ffi.PipelineCfg(S, ni, fa, ct, gh, float(self.prior(p)), (C.c_float * 3)(*thr),
-                               int(round(float(p))) if self.wt else 0, 1 if self.osd0 else 0,
-                               1 if self.skip_inactive else 0, 1 if self.early_stop else 0, self.osd_order)
+                               int(round(float(p))) if self.wt else 0, 1 if (self.osd0 or lsd is not None) else 0,
+                               1 if self.skip_inactive else 0, 1 if self.early_stop else 0, self.osd_order,
+                               1 if lsd is not None else 0, lsd.max_cols if lsd is not None else 0,
+                               lsd.max_checks if lsd is not None else 0)
         return cfg, (ni, fa, ct, gh)
 
     def run(self, batch_size, p, noise=None, want_flags=True, want_diff=True, want_counters=False):
@@ -430,6 +443,7 @@ class BP_BSC_Model:
         self._osd_basis = None          # set by BP2_OSD_Model
         self._osd_pivot = None
         self._osd_order = 0
+        self._lsd = None                # set by BP2_OSD_Model with an LSD_Decoder
         self.last_counters = None
 
     def llr_const(self, p):
@@ -459,12 +473,18 @@ class BP_BSC_Model:
                 raise ValueError(f"noise must have shape [{B},{self.n}], got {keep.shape}")
             nz = keep.t2()
         d = self.decoder
-        _ffi.call("fbgnn_bsc_pipeline_run_ex", g.handle, lg.handle if lg is not None else None,
-                  CN_TYPES[d.cn_type], d.num_iter, d.normalization_factor, float(self.llr_const(p)),
-                  float(np.float32(p)), self.seed, self.next_frame, B, nz, flags.ptr, counters,
-                  self._osd_basis.handle if self._osd_basis is not None else None,
-                  self._osd_pivot.ctypes.data_as(C.POINTER(C.c_int32)) if self._osd_pivot is not None else None,
-                  self._osd_order)
+        if self._lsd is not None:
+            _ffi.call("fbgnn_bsc_pipeline_run_lsd", g.handle, lg.handle if lg is not None else None,
+                      CN_TYPES[d.cn_type], d.num_iter, d.normalization_factor, float(self.llr_const(p)),
+                      float(np.float32(p)), self.seed, self.next_frame, B, nz, flags.ptr, counters,
+                      self._lsd.max_cols, self._lsd.max_checks)
+        else:
+            _ffi.call("fbgnn_bsc_pipeline_run_ex", g.handle, lg.handle if lg is not None else None,
+                      CN_TYPES[d.cn_type], d.num_iter, d.normalization_factor, float(self.llr_const(p)),
+                      float(np.float32(p)), self.seed, self.next_frame, B, nz, flags.ptr, counters,
+                      self._osd_basis.handle if self._osd_basis is not None else None,
+                      self._osd_pivot.ctypes.data_as(C.POINTER(C.c_int32)) if self._osd_pivot is not None else None,
+                      self._osd_order)
         if noise is None:
             self.next_frame += B
         self.last_counters = np.array(list(counters), np.int64) if want_counters else None

@@ -242,6 +242,20 @@ int fbgnn_osd0_decode(fbgnn_graph *basis, int64_t B, fbgnn_tensor2 llr, fbgnn_te
 int fbgnn_osd_decode(fbgnn_graph *basis, int32_t order, int64_t B, fbgnn_tensor2 llr, fbgnn_tensor2 synd,
                      fbgnn_tensor2 e_hat);
 
+/* Localised statistics decoding of order 0 (LSD-0; Hillmann, Berent, Quintavalle, Eisert, Wille, Roffe, 2024; the
+ * `ldpc` package's BpLsdDecoder) on any parity-check matrix `pcm` (R rows; the full hx / hz or an OSD basis).  Clusters
+ * grow around the unsatisfied checks, one column per invalid cluster and round, taking the least reliable column
+ * (ascending llr, ties by index, -0.0 before +0.0) next to the cluster; clusters that meet are united; a cluster stops
+ * growing once its syndrome lies in the span of its columns, and each is then solved as OSD-0 would solve it
+ * (csrc/fbgnn_lsd.cuh and DESIGN.md §4 give the exact definition).  llr float32 (b, v), synd uint8 (row, b) over all R
+ * rows, e_hat uint8 (b, v) (optional: NULL ptr skips it).  max_cols / max_checks bound the columns and checks of all clusters of a frame together
+ * (0 = defaults 256 / 256; limits 512 / 512, outside [1, limit]: FBGNN_E_INVALID).  status (optional, device uint8
+ * [B]): 0 solved (pcm e_hat = synd), 1 abandoned over budget, 2 abandoned because the syndrome is outside the column
+ * space of pcm; an abandoned frame gets e_hat = 0.  One CTA per frame; works for every graph fbgnn_graph_create
+ * accepts. */
+int fbgnn_lsd_decode(fbgnn_graph *pcm, int32_t max_cols, int32_t max_checks, int64_t B, fbgnn_tensor2 llr,
+                     fbgnn_tensor2 synd, fbgnn_tensor2 e_hat, uint8_t *status);
+
 /* ---- feedback GNN --------------------------------------------------------------------- */
 /* Weights in Keras get_weights() order, host float32 pointers (copied); bias pointers may
  * be NULL when use_bias is False.  Shapes: W0[H,3] b0[3] W1x[4,H] b1x[H] W2x[H,M] b2x[M]
@@ -327,6 +341,11 @@ typedef struct {
                                /*    to the reference in general -- a converged frame keeps its first converged state)  */
     int32_t osd_order;         /* with osd0: 0 = OSD-0, lam in [1, 65535] = OSD-CS of order lam (fbgnn_osd_decode),     */
                                /*    the same order on both sides (basis_x with osd_llrz, basis_z with osd_llrx)       */
+    int32_t lsd;               /* with osd0: 1 = re-solve the frames still mismatching with LSD-0 (fbgnn_lsd_decode)   */
+                               /*    instead of OSD, on each side's full matrix (hx with osd_llrz and the full         */
+                               /*    syndrome_x, hz with osd_llrx); no fbgnn_code_set_basis needed; a side LSD-0       */
+                               /*    abandons keeps its BP decision                                                     */
+    int32_t lsd_max_cols, lsd_max_checks;   /* LSD-0 budgets (0 = defaults), as fbgnn_lsd_decode                       */
 } fbgnn_pipeline_cfg;
 
 /* Sandwich_BP_GNN_Evaluation_Model.call on global frames [first_frame, first_frame+B).
@@ -369,6 +388,12 @@ int fbgnn_bsc_pipeline_run_ex(fbgnn_graph *graph, fbgnn_graph *logical, int32_t 
                               uint64_t first_frame, int64_t B, fbgnn_tensor2 noise, uint8_t *flags,
                               int64_t *counters, fbgnn_graph *osd_basis, const int32_t *osd_pivot,
                               int32_t osd_order);
+/* The same with LSD-0 (fbgnn_lsd_decode, sign -1: the binary decoder's logits) on `graph` itself for the failed frames,
+ * with the budgets max_cols / max_checks (0 = defaults); an abandoned frame keeps its BP decision. */
+int fbgnn_bsc_pipeline_run_lsd(fbgnn_graph *graph, fbgnn_graph *logical, int32_t cn_type,
+                               int32_t num_iter, float factor, float llr_const, float p, uint64_t seed,
+                               uint64_t first_frame, int64_t B, fbgnn_tensor2 noise, uint8_t *flags,
+                               int64_t *counters, int32_t max_cols, int32_t max_checks);
 
 /* ---- multi-GPU: the one collective of the path (SURVEY.md 8(e)) ------------------------- */
 /* Monte-Carlo frames shard across the GPUs of a box by global frame id; nothing but the counters is
