@@ -358,19 +358,12 @@ FB_HD float fb_sfu_vn_msg(float num, float a, float u, float corr) {      /* u =
  * x + log(1 - t), each rounded to float32 where the reference rounds them (at the magnitude of x), then subtracted --
  * the reference's phi with its float32 cancellation for large x reproduced, which the decoder's error rates depend
  * on (profiles/r02_ler_phi_forms.txt).  Never negative: lg2 >= 0 on [1, 2], <= 0 on (0, 1], and the two FMAs round
- * monotonically.  FB_SFU_PHI_STABLE (lab) subtracts the logarithms first: the better conditioned log((1+t)/(1-t)). */
-#ifndef FB_SFU_PHI_STABLE
-#define FB_SFU_PHI_STABLE 0
-#endif
+ * monotonically. */
 FB_HD float fb_sfu_phi_open(float x) {
     float t = fb_sfu_exp2s(x, -FB_LOG2E);
     float la = fb_mufu_lg2(FB_ADD(1.0f, t));
     float lb = fb_mufu_lg2(FB_FMAX(FB_SUB(1.0f, t), 1.1920928955078125e-7f));
-#if FB_SFU_PHI_STABLE
-    return FB_MUL(FB_SUB(la, lb), FB_LN2);
-#else
     return FB_SUB(FB_FMA(la, FB_LN2, x), FB_FMA(lb, FB_LN2, x));
-#endif
 }
 FB_HD float fb_sfu_phi4_open(float x) { return fb_sfu_phi_open(x); }
 FB_HD float fb_sfu_phi2_open(float x) { return fb_sfu_phi_open(x); }
@@ -445,11 +438,7 @@ __device__ __forceinline__ float2 fb_sfu_phi_open2(float2 x) {
     const float2 sa = FB_ADD2(fb2s(1.0f), t), sb = FB_SUB2(fb2s(1.0f), t);
     const float2 la = fb2(fb_mufu_lg2(sa.x), fb_mufu_lg2(sa.y));
     const float2 lb = fb2(fb_mufu_lg2(FB_FMAX(sb.x, 1.1920928955078125e-7f)), fb_mufu_lg2(FB_FMAX(sb.y, 1.1920928955078125e-7f)));
-#if FB_SFU_PHI_STABLE
-    return FB_MUL2(FB_SUB2(la, lb), fb2s(FB_LN2));
-#else
     return FB_SUB2(FB_FMA2(la, fb2s(FB_LN2), x), FB_FMA2(lb, fb2s(FB_LN2), x));
-#endif
 }
 __device__ __forceinline__ float2 fb_sfu_tanhf2(float2 x) {
     const float2 ax = fb2(FB_FMIN(FB_I2F(FB_F2I(x.x) & 0x7fffffff), 10.0f), FB_FMIN(FB_I2F(FB_F2I(x.y) & 0x7fffffff), 10.0f));

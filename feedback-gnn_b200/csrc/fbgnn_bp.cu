@@ -19,8 +19,7 @@ static int pick_threads(int n_items_a, int n_items_b) {
 static size_t bp4_smem(const SideDev &X, const SideDev &Z, bool const_prior, bool iter_logits) {
     const size_t np = (size_t)pad4(X.n);
     return sizeof(float) * ((size_t)X.E + Z.E + ((const_prior ? 2 : 3) + (iter_logits ? 2 : 0)) * np) +
-           (size_t)pad16(X.m + Z.m) + 2 * (((size_t)X.n + 1) & ~(size_t)1) + X.n + 16 +
-           (FBGNN_SMEM_TABLES ? 2 * ((size_t)X.E + Z.E) + 32 : 0);
+           (size_t)pad16(X.m + Z.m) + 2 * (((size_t)X.n + 1) & ~(size_t)1) + X.n + 16;
 }
 
 template <bool CP, int DV, int DC, typename MATH, bool FPX>
@@ -36,9 +35,9 @@ template <int DV, int DC>
 static int launch_bp4_m(fbgnn_ctx *ctx, const Bp4Args &a, int64_t grid, size_t smem, int threads, bool cp) {
     // fixed-point exit: regular graph, boxplus-phi, long runs (the bookkeeping costs ~5 % per unsaturated iteration
     // and a 16-iteration stage does not converge-and-saturate in time).  Valid in both arithmetics: the saturation
-    // constants are exact in each.
-    static const int fpx_min_iter = getenv("FBGNN_FPX_MIN_ITER") ? atoi(getenv("FBGNN_FPX_MIN_ITER")) : 32;   // lab knob
-    const bool fpx = DV > 0 && a.cn_type == 0 && a.num_iter >= fpx_min_iter && !a.iter_logits.ptr;
+    // constants are exact in each.  From 32 iterations on: with the exit in the 16-iteration stages too, the headline
+    // pipeline measured 430.7 k instead of 441.1 k frames/s on B200 (profiles/r02_lab_k_bp4_variants.txt).
+    const bool fpx = DV > 0 && a.cn_type == 0 && a.num_iter >= 32 && !a.iter_logits.ptr;
     if (ctx->math_mode == FBGNN_MATH_SFU) {
         if (fpx)
             return cp ? launch_bp4_t<true, DV, DC, MathSfu, true>(ctx, a, grid, smem, threads)
@@ -105,11 +104,9 @@ static int launch_bp4_cluster(fbgnn_ctx *ctx, const Bp4Args &a, int64_t frames, 
     const SideDev &X = a.X, &Z = a.Z;
     if (!X.h_vn_ptr || !Z.h_vn_ptr || a.iter_logits.ptr || a.iters_out || a.rows_x_ptr) return 1;
     const int n = X.n, mt = X.m + Z.m;
-    // Smallest cluster whose CTAs fit; FBGNN_BP4_CLUSTER=<C> (lab knob) starts the search at C.  Measured on the
-    // [[7688,50]] code (profiles/r02_cluster_vs_gstate.txt).
-    int c_first = 4;                   // 4 CTAs per frame measured best (2: too few warps per SM; 8: barrier cost)
-    if (const char *e = getenv("FBGNN_BP4_CLUSTER")) c_first = std::max(2, std::min(CL_MAX, atoi(e)));
-    for (int C = c_first; C <= CL_MAX; C *= 2) {
+    // Smallest cluster of at least 4 CTAs whose CTAs fit: 4 CTAs per frame measured best on the [[7688,50]] code (2: too
+    // few warps per SM; 8: barrier cost; profiles/r02_cluster_vs_gstate.txt).
+    for (int C = 4; C <= CL_MAX; C *= 2) {
         ClusterPart P{};
         P.C = C;
         for (int r = 0; r <= C; r++) {
@@ -138,10 +135,8 @@ int launch_bp4(fbgnn_ctx *ctx, const Bp4Args &a_in, int64_t grid) {
     Bp4Args a = a_in;
     a.stats = ctx->stats;
     const bool cp = a.llr.ptr == nullptr;
-    static const size_t smem_pad = getenv("FBGNN_BP4_SMEM_PAD") ? (size_t)atoi(getenv("FBGNN_BP4_SMEM_PAD")) : 0;   // lab knob
-    const size_t smem = bp4_smem(a.X, a.Z, cp, a.iter_logits.ptr != nullptr) + smem_pad;
-    int threads = pick_threads(a.X.n, a.X.m + a.Z.m);
-    if (const char *t = getenv("FBGNN_BP4_THREADS")) threads = std::max(32, std::min(512, atoi(t) / 32 * 32));   // lab knob
+    const size_t smem = bp4_smem(a.X, a.Z, cp, a.iter_logits.ptr != nullptr);
+    const int threads = pick_threads(a.X.n, a.X.m + a.Z.m);
     if (smem > ctx->smem_optin) {
         // Larger than one SM: a thread-block cluster with the messages in distributed shared memory, or the kernel whose
         // state lives in HBM / L2.  Measured on the [[7688,50]] code (profiles/r02_cluster_vs_gstate.txt): the cluster of

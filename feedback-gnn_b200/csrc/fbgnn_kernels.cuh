@@ -65,7 +65,6 @@ __device__ __forceinline__ float u01(uint32_t r) { return (float)(r >> 8) * 5.96
 // measured on the hardware), both carry the reference's saturation constants exactly, and the published logical
 // error rates are reproduced in both (tests/test_gpu_sfu.py).
 struct MathExact {
-    static constexpr bool kSaturationShortcuts = true;
     static constexpr bool kSharedVnCorr = false;       // the reference's per-edge logaddexp
     static constexpr bool kPaired = false;             // FP32-pipe-bound: packed FP32 loses here (see WSmem)
     static __device__ __forceinline__ float softplus(float x) { return fb_softplusf(x); }
@@ -91,7 +90,6 @@ struct MathExact {
 };
 
 struct MathSfu {
-    static constexpr bool kSaturationShortcuts = true;
     static constexpr bool kSharedVnCorr = true;        // fb_math.h fb_sfu_vn_corr: one correction term per side and variable
     static __device__ __forceinline__ float softplus(float x) { return fb_sfu_softplusf(x); }
     static __device__ __forceinline__ float logaddexp(float a, float b) { return fb_sfu_logaddexpf(a, b); }
@@ -110,38 +108,6 @@ struct MathSfu {
     static __device__ __forceinline__ float2 tanh2(float2 x) { return fb_sfu_tanhf2(x); }
 };
 
-// Lab knobs (make lab ..., tools/lab_bench.py): compile-time experiments, all bit-exact.  Measured on B200
-// (profiles/r02_lab_k_bp4_variants.txt, headline pipeline): group 1 / 2 / 3 / 6 = 184.0 / 188.2 / 189.3 / 185.0 k
-// frames/s with the lean cores, 182.2 k without them.
-#ifndef FBGNN_PHI_GROUP
-#define FBGNN_PHI_GROUP 3          // phi call sites of a check evaluated under one warp vote: the G polynomial chains
-                                   // interleave (the single-site form leaves the warp latency-bound on one Horner chain)
-#endif
-#ifndef FBGNN_LAE_GROUP
-#define FBGNN_LAE_GROUP 3          // logaddexp sites of a variable node evaluated under one warp vote (3 = per side, 6 = all)
-#endif
-#ifndef FBGNN_SIGNBITS
-#define FBGNN_SIGNBITS 1           // quaternary check nodes: sign parity as an XOR of the message words (lab: 0 = comparisons)
-#endif
-#ifndef FBGNN_FPX_START
-#define FBGNN_FPX_START 6          // first iteration with a fixed-point test
-#endif
-#ifndef FBGNN_FPX_STRIDE
-#define FBGNN_FPX_STRIDE 3         // iterations between two fixed-point tests of the first stage (1 / 2 / 3 / 4: 414 / 434 / 441 / 436 k frames/s)
-#endif
-#ifndef FBGNN_SMEM_TABLES
-#define FBGNN_SMEM_TABLES 0        // lab: check-side edge tables in shared memory instead of global memory behind L1
-#endif
-#ifndef FBGNN_UNIFORM
-#define FBGNN_UNIFORM 1            // regular fast path: warp-uniform node loops, full-mask votes
-#endif
-#ifndef FBGNN_VOTE
-#define FBGNN_VOTE 1               // 0 (lab): evaluate always, select afterwards -- no warp vote / branch
-#endif
-#ifndef FBGNN_LEAN
-#define FBGNN_LEAN 1               // no clamps inside the voted evaluations (identity for the lanes that use them)
-#endif
-
 // ------------------------------------------------------------------ saturated fast paths
 // Value-dependent shortcuts that return exactly what the full evaluation returns:
 //   phi(x) = phi(clip_hi) = +0          for x >= 16.635532,
@@ -151,19 +117,15 @@ struct MathSfu {
 // Once a frame has converged nearly every message sits in these regimes; a warp whose lanes are all
 // saturated skips the polynomial evaluation altogether (the vote only decides whether the full path
 // is executed, never which value a lane takes).
+// Inside a voted evaluation only the lanes with 8.5e-8 < x < 16.635532 keep the value: no clamp needed.
 template <typename MATH, bool PHI4>
-__device__ __forceinline__ float phi_eval(float x) {
-    // inside a voted evaluation only the lanes with 8.5e-8 < x < 16.635532 keep the value: no clamp needed
-    if (FBGNN_LEAN && MATH::kSaturationShortcuts) return PHI4 ? MATH::phi4_open(x) : MATH::phi2_open(x);
-    return PHI4 ? MATH::phi4(x) : MATH::phi2(x);
-}
+__device__ __forceinline__ float phi_eval(float x) { return PHI4 ? MATH::phi4_open(x) : MATH::phi2_open(x); }
 
 template <typename MATH, bool PHI4>
 __device__ __forceinline__ float phi_sat(float x) {
-    if (!MATH::kSaturationShortcuts) return PHI4 ? MATH::phi4(x) : MATH::phi2(x);
     const bool hi = x >= FB_PHI_CLIP_HI, lo = x <= FB_PHI_CLIP_LO;
     float r = hi ? 0.0f : FB_PHI_CLIP_HI;
-    if (!FBGNN_VOTE || __any_sync(__activemask(), !(hi || lo))) {
+    if (__any_sync(__activemask(), !(hi || lo))) {
         const float f = phi_eval<MATH, PHI4>(x);
         r = (hi || lo) ? r : f;
     }
@@ -174,11 +136,6 @@ __device__ __forceinline__ float phi_sat(float x) {
 // all G when any lane needs any of them.  Values are those of phi_sat.
 template <typename MATH, bool PHI4, int G, bool FULL = false>
 __device__ __forceinline__ void phi_sat_group(const float x[G], float r[G]) {
-    if (!MATH::kSaturationShortcuts) {
-#pragma unroll
-        for (int k = 0; k < G; k++) r[k] = PHI4 ? MATH::phi4(x[k]) : MATH::phi2(x[k]);
-        return;
-    }
     bool sat[G], need = false;
 #pragma unroll
     for (int k = 0; k < G; k++) {
@@ -187,9 +144,9 @@ __device__ __forceinline__ void phi_sat_group(const float x[G], float r[G]) {
         r[k] = hi ? 0.0f : FB_PHI_CLIP_HI;
         need = need || !sat[k];
     }
-    if (!FBGNN_VOTE || __any_sync(FULL ? 0xffffffffu : __activemask(), need)) {
+    if (__any_sync(FULL ? 0xffffffffu : __activemask(), need)) {
         int k0 = 0;
-        if constexpr (MATH::kPaired && FBGNN_LEAN) {         // sites 2i, 2i+1 as one float2 evaluation (odd G: the last alone)
+        if constexpr (MATH::kPaired) {         // sites 2i, 2i+1 as one float2 evaluation (odd G: the last alone)
 #pragma unroll
             for (; k0 + 1 < G; k0 += 2) {
                 const float2 f = MATH::phi_open2(make_float2(x[k0], x[k0 + 1]));
@@ -207,17 +164,11 @@ __device__ __forceinline__ void phi_sat_group(const float x[G], float r[G]) {
 
 template <typename MATH>
 __device__ __forceinline__ float logaddexp_sat(float a, float b) {
-    if (!MATH::kSaturationShortcuts) return MATH::logaddexp(a, b);
     const float mx = fmaxf(a, b), mn = fminf(a, b);
     const bool sat = FB_SUB(mn, mx) < -17.5f;
     float r = FB_ADD(0.0f, mx);
-    if (!FBGNN_VOTE || __any_sync(__activemask(), !sat)) {
-        float f;
-        if (FBGNN_LEAN) {           // exp without its clamp: d >= -17.5 on the lanes that keep f
-            f = MATH::logaddexp_open(mx, FB_SUB(mn, mx));
-        } else {
-            f = MATH::logaddexp(a, b);
-        }
+    if (__any_sync(__activemask(), !sat)) {
+        const float f = MATH::logaddexp_open(mx, FB_SUB(mn, mx));     // exp without its clamp: d >= -17.5 on the lanes that keep f
         r = sat ? r : f;
     }
     return r;
@@ -235,7 +186,7 @@ __device__ __forceinline__ void logaddexp_sat_group(const float a[G], const floa
         r[k] = FB_ADD(0.0f, mx[k]);
         need = need || !(d[k] < -17.5f);
     }
-    if (!FBGNN_VOTE || __any_sync(0xffffffffu, need)) {
+    if (__any_sync(0xffffffffu, need)) {
 #pragma unroll
         for (int k = 0; k < G; k++) {
             const float f = MATH::logaddexp_open(mx[k], d[k]);
@@ -259,7 +210,7 @@ __device__ __forceinline__ void vn_corr_pair(float lx, float ly, float lz, float
     }
     const bool satx = dx < -17.5f, satz = dz < -17.5f;
     cx = 0.0f; cz = 0.0f;
-    if (!FBGNN_VOTE || __any_sync(FULL ? 0xffffffffu : __activemask(), !(satx && satz))) {
+    if (__any_sync(FULL ? 0xffffffffu : __activemask(), !(satx && satz))) {
         float fx, fz;
         if constexpr (PAIRED) {
             const float2 f = MATH::logaddexp_open2(make_float2(0.0f, 0.0f), make_float2(dx, dz));
@@ -381,12 +332,15 @@ __device__ __forceinline__ bool cn_phi_regular(const idx_t *__restrict__ cn_edge
     // making: never -0.0 (x - y rounds to +0 when it is zero) and never NaN, so "m < 0" IS the sign bit and the parity
     // of the signs is an XOR of the message words (SIGNBITS).  The binary decoder keeps the comparisons: its messages
     // can be scaled by negative edge weights, which makes -0.0 reachable, and sign(-0.0) counts as +1 in the reference.
-    constexpr bool SIGNBITS = PHI4 && FBGNN_SIGNBITS;
+    constexpr bool SIGNBITS = PHI4;
     uint32_t neg = 0, word[DC], pw = (uint32_t)synd_bit << 31;
     int par = synd_bit;
 #pragma unroll
     for (int k = 0; k < DC; k++) e[k] = cn_edge[c * DC + k];
-    constexpr int GRP = (FBGNN_PHI_GROUP > 0 && DC % FBGNN_PHI_GROUP == 0) ? FBGNN_PHI_GROUP : (DC % 2 == 0 ? 2 : 1);
+    // phi call sites evaluated under one warp vote: the GRP polynomial chains interleave (the single-site form leaves the
+    // warp latency-bound on one Horner chain).  Measured on B200 (profiles/r02_lab_k_bp4_variants.txt, headline
+    // pipeline): group 1 / 2 / 3 / 6 = 184.0 / 188.2 / 189.3 / 185.0 k frames/s.
+    constexpr int GRP = DC % 3 == 0 ? 3 : (DC % 2 == 0 ? 2 : 1);
     float xin[DC];
 #pragma unroll
     for (int k = 0; k < DC; k++) {
@@ -508,9 +462,11 @@ __device__ __forceinline__ void vn_update_regular(int v, float *mx, float *mz, f
         }
         return;
     }
-    if (FULL && MATH::kSaturationShortcuts && FBGNN_LEAN) {
-        // the 2 DV logaddexp sites under FBGNN_LAE_GROUP-sized votes (same values as one vote per site)
-        constexpr int LG = (FBGNN_LAE_GROUP > 0 && (2 * DV) % FBGNN_LAE_GROUP == 0) ? FBGNN_LAE_GROUP : DV;
+    if (FULL) {
+        // the 2 DV logaddexp sites under votes of 3 sites if 3 divides 2 DV, else of DV sites (same values as one vote per
+        // site).  Measured on B200 when the SFU arithmetic still took this path (profiles/r02_lab_k_bp4_variants.txt):
+        // groups of 3 / 6 / 2 = 316.4 / 312.5 / 315.4 k frames/s.
+        constexpr int LG = (2 * DV) % 3 == 0 ? 3 : DV;
         float p[2 * DV], q[2 * DV], r[2 * DV];
 #pragma unroll
         for (int k = 0; k < DV; k++) {
@@ -694,14 +650,7 @@ static __global__ void __launch_bounds__(512, (MATH::kPaired && DV > 0 && DV <= 
     float *mz = mx + X.E, *scr2 = mz + Z.E;
     uint16_t *rec = GSTATE ? (uint16_t *)(sbx + mp) : (uint16_t *)(scr2 + (a.iter_logits.ptr ? 2 * np : 0));
     uint8_t *dec = (uint8_t *)(rec + ((n + 1) & ~1));
-#if FBGNN_SMEM_TABLES       // lab: the check-side edge tables copied into shared memory (north star "edge lists in shared memory")
-    idx_t *tabx = (idx_t *)(dec + ((n + 15) & ~15)), *tabz = tabx + X.E;
-    for (int e = tid; e < X.E; e += T) tabx[e] = X.cn_edge[e];
-    for (int e = tid; e < Z.E; e += T) tabz[e] = Z.cn_edge[e];
-    const idx_t *cn_edge_x = tabx, *cn_edge_z = tabz;
-#else
     const idx_t *cn_edge_x = X.cn_edge, *cn_edge_z = Z.cn_edge;
-#endif
 
     // per-frame inputs: the pipeline's workspace rows are 16-byte aligned blocks -> two bulk-async (TMA) copies posted by one
     // thread, overlapped with the clearing of the messages; the layer API's strided views are read element by element
@@ -729,20 +678,21 @@ static __global__ void __launch_bounds__(512, (MATH::kPaired && DV > 0 && DV <= 
     __syncthreads();
 
     const bool fast = DV > 0 && a.cn_type == 0;     // regular graph + boxplus-phi: unrolled path
-    constexpr bool uniform = FBGNN_UNIFORM != 0;    // the launchers only use multiples of 32 threads
-    // Fixed-point exit (exact arithmetic only): once an iteration reproduces every message bit for bit
+    // Fixed-point exit: once an iteration reproduces every message bit for bit
     // the remaining iterations are no-ops, so they are skipped -- the outputs are unchanged by construction.
     // Only worth its bookkeeping for long runs (the 64-iteration first stage), and never before iteration 6.
-    const bool fp_exit = FPX && fast && MATH::kSaturationShortcuts && !a.iter_logits.ptr;
+    const bool fp_exit = FPX && fast && !a.iter_logits.ptr;
     const int sat_bits = __float_as_int(FB_MUL(FB_PHI_CLIP_HI, a.factor)) & 0x7fffffff;   // |phi(clip_lo) * factor|
     int it_done = a.num_iter;
     for (int it = 0; it < a.num_iter; it++) {
         if (a.iter_logits.ptr) bp4_iter_logits<CONST_PRIOR, MATH>(a, mx, mz, pri, scr2, dec, b, it);
-        // the fixed-point test runs every FBGNN_FPX_STRIDE-th iteration: a later test only delays the exit by no-op iterations
-        uint16_t *recp = (fp_exit && it >= FBGNN_FPX_START && (it % FBGNN_FPX_STRIDE) == 0) ? rec : nullptr;
+        // the fixed-point test runs every third iteration: a later test only delays the exit by no-op iterations.  Measured
+        // on B200 (profiles/r02_lab_k_bp4_variants.txt): stride 1 / 2 / 3 / 4 = 414 / 434 / 441 / 436 k frames/s.
+        uint16_t *recp = (fp_exit && it >= 6 && (it % 3) == 0) ? rec : nullptr;
         // variable nodes (decoding_q.py:227-275)
-        if (DV > 0 && uniform) {
-            // whole warps take the full-mask instantiation, the ragged last warp the activemask one
+        if (DV > 0) {
+            // whole warps take the full-mask instantiation, the ragged last warp the activemask one (the launchers only use
+            // multiples of 32 threads)
             for (int v = tid; v < n; v += T) {
                 const float px = CONST_PRIOR ? a.prior : pri[v];
                 const float py = CONST_PRIOR ? a.prior : pri[np + v];
@@ -755,10 +705,6 @@ static __global__ void __launch_bounds__(512, (MATH::kPaired && DV > 0 && DV <= 
             const float px = CONST_PRIOR ? a.prior : pri[v];
             const float py = CONST_PRIOR ? a.prior : pri[np + v];
             const float pz = CONST_PRIOR ? a.prior : pri[2 * np + v];
-            if (DV > 0) {
-                vn_update_regular<(DV > 0 ? DV : 1), MATH, FPX>(v, mx, mz, px, py, pz, recp, sat_bits);
-                continue;
-            }
             const int x0 = X.vn_ptr[v], x1 = X.vn_ptr[v + 1], z0 = Z.vn_ptr[v], z1 = Z.vn_ptr[v + 1];
             float Sx = 0.0f, Sz = 0.0f;
             for (int e = x0; e < x1; e++) Sx = FB_ADD(Sx, mx[e]);
@@ -786,7 +732,7 @@ static __global__ void __launch_bounds__(512, (MATH::kPaired && DV > 0 && DV <= 
         __syncthreads();
         // check nodes of both sides as one index space
         bool stable = true;
-        if (fast && uniform) {
+        if (fast) {
             const int mt = X.m + Z.m;
             for (int c = tid; c < mt; c += T) {
                 const bool isx = c < X.m;
@@ -804,13 +750,8 @@ static __global__ void __launch_bounds__(512, (MATH::kPaired && DV > 0 && DV <= 
             const int cc = isx ? c : c - X.m;
             float *msg = isx ? mx : mz;
             const int sb = isx ? sbx[cc] : sbz[cc];
-            if (fast) {
-                stable &= cn_phi_regular<(DC > 0 ? DC : 1), (DV > 0 ? DV : 1), true, MATH, FPX>(
-                    isx ? cn_edge_x : cn_edge_z, cc, msg, sb, a.factor, recp, isx ? 0 : DV);
-            } else {
-                const SideDev &S = isx ? X : Z;
-                cn_update_one<true, MATH>(S.cn_edge, S.cn_ptr[cc], S.cn_ptr[cc + 1], msg, sb, a.cn_type, a.factor);
-            }
+            const SideDev &S = isx ? X : Z;
+            cn_update_one<true, MATH>(S.cn_edge, S.cn_ptr[cc], S.cn_ptr[cc + 1], msg, sb, a.cn_type, a.factor);
         }
         if (FPX && recp) {
             if (__syncthreads_and(stable)) { it_done = it + 1; break; }
@@ -1049,10 +990,6 @@ static __global__ void __launch_bounds__(512) k_bp2(const Bp2Args a) {
 }
 
 // ------------------------------------------------------------------ feedback GNN ------
-#ifndef FBGNN_GNN_UNROLL
-#define FBGNN_GNN_UNROLL 1            // hidden units of the regular path per loop trip (lab knob)
-#endif
-constexpr int kGnnUnroll = FBGNN_GNN_UNROLL;
 struct GnnArgs {
     SideDev X, Z;
     const float *weights;               // packed, see GnnLayout
@@ -1118,8 +1055,8 @@ struct WSmem {
 // The two sides share ONE copy of the inner loop (side loop not unrolled) and the loop over hidden
 // units is unrolled by two only: the hot loop body stays a few KB, inside the instruction cache.
 // Requires H % 4 == 0 and M % 4 == 0.
-template <int H, int M, int DV, bool TANH_BIAS, bool FACT, typename MATH, typename WSRC>
-__device__ __forceinline__ void gnn_body(const GnnArgs &a, const WSRC w) {
+template <int H, int M, int DV, bool TANH_BIAS, bool FACT, typename MATH>
+__device__ __forceinline__ void gnn_body(const GnnArgs &a, const WSmem w) {
     typedef GnnLayout<H, M> Lay;
     static_assert(FACT || DV == 0, "the per-edge form is only built for the generic degree path");
     constexpr int NE = DV > 0 ? DV : 1;
@@ -1148,7 +1085,7 @@ __device__ __forceinline__ void gnn_body(const GnnArgs &a, const WSRC w) {
             }
 #pragma unroll
             for (int i = 0; i < M; i++) { rx[i] = 0.0f; rz[i] = 0.0f; }
-#pragma unroll kGnnUnroll
+#pragma unroll 1
             for (int j = 0; j < H; j++) {
                 const float4 wx = w.ld4(Lay::W1tx + 4 * j), wz = w.ld4(Lay::W1tz + 4 * j);
                 const float bx = w.ld(Lay::b1x + j), bz = w.ld(Lay::b1z + j);
@@ -1195,20 +1132,11 @@ __device__ __forceinline__ void gnn_body(const GnnArgs &a, const WSRC w) {
             const int oW2 = side ? Lay::W2z : Lay::W2x, ob2 = side ? Lay::b2z : Lay::b2x;
             const View2<const float> &logit = side ? a.logit_hz : a.logit_hx;
             const View2<const uint8_t> &synd = side ? a.sz : a.sx;
-            const int e0 = DV > 0 ? v * DV : S.vn_ptr[v], e1 = DV > 0 ? e0 + DV : S.vn_ptr[v + 1];
+            const int e0 = S.vn_ptr[v], e1 = S.vn_ptr[v + 1];
             float red[M];
 #pragma unroll
             for (int i = 0; i < M; i++) red[i] = 0.0f;
             if (FACT) {
-                float hc[NE];
-                if (DV > 0) {
-#pragma unroll
-                    for (int k = 0; k < NE; k++) {
-                        const int c = S.vn_cn[e0 + k];
-                        const float lg = logit(c, b);
-                        hc[k] = synd(c, b) ? -lg : lg;
-                    }
-                }
 #pragma unroll 2
                 for (int j = 0; j < H; j++) {
                     // features [h_cn, Lx, Ly, Lz]: the per-variable terms first, the check term last
@@ -1216,26 +1144,13 @@ __device__ __forceinline__ void gnn_body(const GnnArgs &a, const WSRC w) {
                                               FB_FMA(f2, w.ld(oW1 + 2 * H + j), FB_FMA(f1, w.ld(oW1 + H + j), 0.0f)));
                     const float w0 = w.ld(oW1 + j), bj = w.ld(ob1 + j);
                     float hs = 0.0f;
-                    if (DV > 0) {
-                        float hv[NE];
-#pragma unroll
-                        for (int k = 0; k < NE; k++) {
-                            float t = FB_FMA(hc[k], w0, base);
-                            if (use_bias) t = FB_ADD(t, bj);
-                            hv[k] = gnn_act<MATH>(act, t);
-                        }
-                        hs = hv[0];
-#pragma unroll
-                        for (int k = 1; k < NE; k++) hs = FB_ADD(hs, hv[k]);
-                    } else {
-                        for (int e = e0; e < e1; e++) {
-                            const int c = S.vn_cn[e];
-                            const float lg = logit(c, b);
-                            float t = FB_FMA(synd(c, b) ? -lg : lg, w0, base);
-                            if (use_bias) t = FB_ADD(t, bj);
-                            const float hv = gnn_act<MATH>(act, t);
-                            hs = (e == e0) ? hv : FB_ADD(hs, hv);
-                        }
+                    for (int e = e0; e < e1; e++) {
+                        const int c = S.vn_cn[e];
+                        const float lg = logit(c, b);
+                        float t = FB_FMA(synd(c, b) ? -lg : lg, w0, base);
+                        if (use_bias) t = FB_ADD(t, bj);
+                        const float hv = gnn_act<MATH>(act, t);
+                        hs = (e == e0) ? hv : FB_ADD(hs, hv);
                     }
 #pragma unroll
                     for (int i = 0; i < M; i += 4) {
@@ -1329,15 +1244,15 @@ __device__ __forceinline__ void gnn_body(const GnnArgs &a, const WSRC w) {
     }
 }
 
-#ifndef FBGNN_GNN_MINBLOCKS
-#define FBGNN_GNN_MINBLOCKS 5         // 96 registers, 5 CTAs / SM: measured best (profiles/r02_lab_k_gnn_variants.txt)
-#endif
+// 96 registers, 5 CTAs / SM, with the regular path's hidden-unit loop not unrolled: measured best on B200
+// (profiles/r02_lab_k_bp4_variants.txt, the k_gnn unroll / occupancy block: 319.5 k frames/s; unrolled by 2: 319.0 k;
+// 4 CTAs / SM: 316.2 k; 6 CTAs / SM: 314.2 k)
 template <int H, int M, int DV, bool TANH_BIAS, bool FACT, typename MATH>
-static __global__ void __launch_bounds__(128, FBGNN_GNN_MINBLOCKS) k_gnn(const GnnArgs a) {
+static __global__ void __launch_bounds__(128, 5) k_gnn(const GnnArgs a) {
     extern __shared__ float wsm[];
     for (int i = threadIdx.x; i < GnnLayout<H, M>::total; i += blockDim.x) wsm[i] = a.weights[i];
     __syncthreads();
-    gnn_body<H, M, DV, TANH_BIAS, FACT, MATH, WSmem>(a, WSmem{wsm});
+    gnn_body<H, M, DV, TANH_BIAS, FACT, MATH>(a, WSmem{wsm});
 }
 
 // ---- feedback GNN with MLPs of any depth (num_mlp_layers != 2; feedback_gnn.py:110-127) ----------------------------

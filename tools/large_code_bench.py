@@ -23,12 +23,8 @@ prior = float(np.log(3 * 0.95 / 0.05))
 res = {"code": code.name, "n": code.N, "frames": B, "iterations": it, "device": ctx.name}
 for arith in ("exact", "sfu"):
     ctx.set_math(arith)
-    for mode in ("cluster2", "cluster4", "cluster8", "gstate"):
-        if mode == "gstate":
-            os.environ["FBGNN_BP4_LARGE"] = "gstate"
-        else:
-            os.environ["FBGNN_BP4_LARGE"] = "cluster"
-            os.environ["FBGNN_BP4_CLUSTER"] = mode[7:]
+    for mode in ("cluster", "gstate"):
+        os.environ["FBGNN_BP4_LARGE"] = mode
         out = dec.decode_device(None, sx, sz, prior=prior)
         ctx.sync()
         ctx.timer_start()
